@@ -55,7 +55,15 @@ def parse_args():
                          "allocates fresh operands for every launch)")
     ap.add_argument("--no-parity", action="store_true",
                     help="skip the pre-timing parity leg (compiled N-GPU steps vs vanilla fp32)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy "
+                         "(its loss; the parameters and momentum buffers it left, sampled), so that "
+                         "two builds can be compared on identical inputs")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "edb" or args.mode == "auto"):
+        ap.error("--dump-outputs covers this backend's data-parallel path (--impl edb, --mode "
+                 "ddp / zero2 / zero3)")
+    return args
 
 
 def measured_peaks():
@@ -374,6 +382,34 @@ def parity_leg(torch, dist, args, cfg, GPT2, step_fn, model, opt, state0, par_ho
     return res
 
 
+def dump_outputs(torch, step_fn, loss, full_shapes, world, rank, out_dir):
+    """The last timed step's results as out_dir/<name>.npy: `loss` (float64) and, in float32, every
+    parameter (`param.<name>`) and optimizer state (`<key>.<name>`) it left, gathered to full size.
+    Tensors above `per` elements are sampled at `per` positions drawn with a fixed seed, which keeps
+    the files under 64 MB in all."""
+    import numpy as np
+    from tools import parity as P
+    params, _, states = step_fn.compiled_func.get_state()
+    tensors = []
+    for name, shape in full_shapes.items():
+        tensors.append((f"param.{name}", params[name], shape))
+        for key, t in states.get(name, {}).items():
+            if isinstance(t, torch.Tensor) and t.dim() > 0:
+                tensors.append((f"{key}.{name}", t, shape))
+    per = min(16384, (60 << 20) // (4 * len(tensors)))
+    arrays = {"loss": np.float64(loss)}
+    for fname, t, shape in tensors:
+        full = P.gather_full(t.detach(), shape, world).flatten()
+        if full.numel() > per:
+            idx = np.sort(np.random.default_rng(0).choice(full.numel(), per, replace=False))
+            full = full[torch.from_numpy(idx).to(full.device)]
+        arrays[fname] = full.float().cpu().numpy()
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        for name, a in arrays.items():
+            np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_edb(args):
     import torch
     import torch.distributed as dist
@@ -410,6 +446,7 @@ def run_edb(args):
     else:
         model = GPT2(cfg).to(device="cuda", dtype=torch.bfloat16)
     opt = torch.optim.SGD(model.parameters(), lr=1e-3, momentum=0.9, foreach=True)
+    full_shapes = {n: p.shape for n, p in model.named_parameters()}
     B, S = args.batch_per_gpu, args.seq
     n_batches = 4
     host = [synthetic_tokens(cfg, B, S, seed=1000 * b + rank) for b in range(n_batches)]
@@ -484,9 +521,11 @@ def run_edb(args):
     torch.cuda.synchronize()
     ms_total, loss_v = timed(args.steps, e2e=False)
     clocks = sampler.stop() if rank == 0 else None
-    ms_e2e, _ = timed(args.steps, e2e=True)
+    ms_e2e, loss_last = timed(args.steps, e2e=True)
     errs = rt.error_flags()
     assert not any(errs), f"collective spin-wait timeouts: {errs}"
+    if args.dump_outputs:
+        dump_outputs(torch, step_fn, loss_last, full_shapes, world, rank, args.dump_outputs)
     gbatch = B * world
     value = gbatch * args.steps / (ms_total / 1e3)
     e2e_value = gbatch * args.steps / (ms_e2e / 1e3)

@@ -35,11 +35,13 @@ def _nvcc():
 
 def _digest(paths):
     h = hashlib.sha256()
+    # paths relative to the repository: a built tree stays current when it is moved or copied
+    rel = lambda s: os.path.relpath(s, ROOT) if os.path.isabs(s) else s
     for p in sorted(paths):
         with open(p, "rb") as f:
-            h.update(p.encode())
+            h.update(rel(p).encode())
             h.update(f.read())
-    h.update(" ".join(NVCC_FLAGS).encode())
+    h.update(" ".join(map(rel, NVCC_FLAGS)).encode())
     return h.hexdigest()
 
 

@@ -39,7 +39,7 @@ def pytest_cmdline_main(config):
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a real B200 (run with -m gpu under gpurun)")
     config.addinivalue_line("markers", "multigpu: needs >= 2 GPUs on the box")
-    config.addinivalue_line("markers", "refonly: needs /root/reference (CPU container only)")
+    config.addinivalue_line("markers", "refonly: needs the reference source tree (EASYDIST_REFERENCE)")
 
 
 @pytest.fixture(scope="session")

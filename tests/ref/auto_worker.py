@@ -57,6 +57,7 @@ def main():
     rank, world = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"])
     mesh_shape = tuple(int(v) for v in os.environ.get("EDB_TEST_MESH", str(world)).split("x"))
     record = os.environ.get("EDB_RECORD", "")
+    record_parity = os.environ.get("EDB_RECORD_PARITY", "")
     planner = os.environ.get("EDB_PLANNER", "GREEDY")
     # recording large plans: rank 0 does the sharding discovery + ILP alone while the others wait
     torch.set_num_threads(int(os.environ.get("EDB_THREADS_RANK0" if rank == 0 else "EDB_THREADS", "1")))
@@ -106,7 +107,7 @@ def main():
             orig = ref_auto.sharding_transform
 
             def mine(fx_module, opt_strategy, state_io_map):
-                if record and rank == 0:
+                if (record or record_parity) and rank == 0:
                     from easydist_b200 import graph_io
                     saved["plan"] = graph_io.dump_bundle(
                         fx_module, opt_strategy,
@@ -186,6 +187,17 @@ def main():
         if record and "plan" in saved:
             with open(record, "w") as f:
                 f.write(saved["plan"])
+        if record_parity:
+            # what tests/test_ref_parity.py compares this backend's lowering of the same plan with,
+            # where the reference is not importable: its comm structure and (a strided sample of)
+            # the outputs of the reference's own lowering
+            import gzip
+            import json
+            sample = lambda o: [float(str(v)) for v in
+                                o.flatten()[::max(1, o.numel() // 256)].numpy()]
+            with gzip.open(record_parity, "wt") as f:
+                json.dump({"bundle": json.loads(saved["plan"]), "hist_ref_same_plan": same,
+                           "ref_outputs": [sample(o) for o in outs_a]}, f, separators=(",", ":"))
     dist.barrier()
     dist.destroy_process_group()
     if not ok:
