@@ -64,18 +64,8 @@ SIGNATURES = {
                                  c_int, _IP, _I64P, _I64P, _I64P, _I64P, c_void_p]),
     "edb_halo_exchange": (c_int, [c_int, c_void_p, c_uint64, c_void_p, _I64P, c_int, c_int, c_int,
                                   c_int, c_void_p]),
-    "edb_symm_guard": (c_int, [c_int, c_void_p]),
     "edb_gemm_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64,
                               c_int64, c_int64, c_int64, c_int, c_int, c_int, c_void_p]),
-    "edb_ag_gemm_bf16": (c_int, [c_int, c_void_p, c_void_p, c_void_p, c_uint64, c_uint64, c_int64,
-                                 c_int64, c_int64, c_int64, c_int64, c_void_p]),
-    "edb_gemm_rs_bf16": (c_int, [c_int, c_void_p, c_uint64, c_void_p, c_void_p, c_int64, c_int64,
-                                 c_int64, c_int64, c_int64, c_int, c_int, c_float, c_int,
-                                 c_void_p]),
-    "edb_gemm_rs_push_bf16": (c_int, [c_int, c_uint64, c_uint64, c_void_p, c_void_p, c_int64, c_int64,
-                                      c_int64, c_int64, c_int64, c_int, c_int, c_void_p]),
-    "edb_rs_finish": (c_int, [c_int, c_int, c_void_p, c_void_p, c_void_p, _I64P, c_float, c_int,
-                              c_void_p]),
     "edb_epoch_barrier": (c_int, [c_int, c_void_p]),
     "edb_all_gather_push": (c_int, [c_int, c_uint64, c_void_p, _I64P, c_int, c_int, c_int, c_void_p]),
     "edb_all_to_all_push": (c_int, [c_int, c_uint64, c_void_p, _I64P, c_int, c_int, c_int, c_int,

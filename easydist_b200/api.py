@@ -94,14 +94,13 @@ def _finish(gm, params, buffers, named_states, args, kwargs, ops, native, io=Non
         lowering.propagate_local_meta(gm, flat)
     # auto-SPMD plan on a 1-D mesh: gathers of parameter shards become prefetches (below)
     auto_pf = (native or fuse_rt is not None) and fuse and auto_io is not None and ranks is not None \
-        and len(ranks) > 1 and os.environ.get("EDB_EPOCH", "1") == "1" \
-        and os.environ.get("EDB_AG_PREFETCH", "1") == "1"
+        and len(ranks) > 1 and os.environ.get("EDB_AG_PREFETCH", "1") == "1"
     bucket = os.environ.get("EDB_BUCKET_COMM", "0") == "1"
     if bucket and not auto_pf:
         # opt-in: changes the communication structure the reference's lowering would produce
         info["bucketed"] = lowering.bucket_small_comm(gm, ops)
         lowering.propagate_local_meta(gm, flat)
-    experimental = [k for k in ("EDB_OVERLAP", "EDB_RS_LANE", "EDB_GEMM_SIDE", "EDB_DEFER_RS")
+    experimental = [k for k in ("EDB_OVERLAP", "EDB_GEMM_SIDE")
                     if os.environ.get(k, "0") == "1"]
     if experimental and native:
         # round-1 advisor finding: kernels whose CTAs wait on other CTAs assume the whole grid is
@@ -169,7 +168,7 @@ def _finish(gm, params, buffers, named_states, args, kwargs, ops, native, io=Non
         # push-protocol collectives need ONE group for the end-of-step barrier: a 1-D mesh / the dp
         # group.  (N-D meshes keep the flag protocol: a barrier per mesh dim would not cover the
         # buffers of the other dims' collectives.)
-        push = ranks is not None and len(ranks) > 1 and os.environ.get("EDB_EPOCH", "1") == "1" \
+        push = ranks is not None and len(ranks) > 1 \
             and os.environ.get("EDB_PUSH_COLL", "1") == "1" and hasattr(ops, "epoch_barrier") \
             and not overlap and _single_group(gm, ops, ranks)
         info["symm_bytes"] = lowering.assign_static_buffers(gm, get_runtime(), ops, push=push)

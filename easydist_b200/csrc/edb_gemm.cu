@@ -331,42 +331,23 @@ __device__ __forceinline__ float gelu_tanh_grad(float x) {
 //   MODE_AG    : B (weights, [N,K] K-major) is sharded S(0) over the group; a few "comm" CTAs pull the
 //                peer shards over NVLink with TMA bulk copies into the local gathered buffer while
 //                the MMA CTAs start on the local shard and pick up chunks as their flags arrive
-//                (all_gather_end -> aten.mm of the sharded graph in one kernel)
-//   MODE_RS    : the partial product C is reduce-scattered over its rows: the epilogue TMA-stores
-//                every tile straight into the owner's receive slot over NVLink (own rows last),
-//                per-chunk flags tell the owner when a source is complete, and the tail of the same
-//                kernel reduces the n slots in rank order with scale + cast
-//                (aten.mm -> reduce_scatter_start in one kernel)
-enum { MODE_PLAIN = 0, MODE_AG = 1, MODE_RS = 2 };
+//                (all_gather_end -> aten.mm of the sharded graph in one kernel).  No handshake with
+//                the peers inside the kernel: an edb_epoch_barrier earlier on the stream made every
+//                member's shard final, and the next barrier comes before anybody overwrites it.
+//                Only the local chunk flags (comm CTAs -> MMA CTAs) remain.
+enum { MODE_PLAIN = 0, MODE_AG = 1 };
 constexpr int kMaxPfItems = 4;
 constexpr int kPfSlots = 12, kPfDepth = 8;  // 16 KiB slots of the prefetch ring / loads in flight
-constexpr int F_TILECNT = 96;  // flag-block words [96,104): per-chunk completion counters
 
 struct FusedArgs {
   FlagCtx f;
-  int n_comm;  // MODE_AG: number of comm CTAs at the end of the grid
+  int n_comm;  // MODE_AG: number of comm CTAs at the start of the grid
   // MODE_AG
   const char* shard_src[kMaxGroup];  // member p's shard (peer mapped); [me] is local
   char* full_dst;                    // local gathered buffer
   int64_t shard_bytes;
   int ag_rows;        // rows of B per shard (N / n)
   int ag_first_tile;  // n-tile containing the first row of my shard
-  // MODE_RS
-  char* recv_base;      // my receive buffer: n slots of chunk_bytes
-  int64_t chunk_bytes;  // (M/n) * N * 2
-  void* rs_dst;
-  float rs_scale;
-  int rs_out_dtype;
-  int tiles_per_chunk;
-  // deferred reduce-scatter: the kernel only pushes its tiles (flag words F_CHUNK + 8 + src) and
-  // records its op number in rs_state[0]; k_rs_finish reduces the slots later (rs_state[1] = the op
-  // number of that reduction, which guards the slots against the next step's pushes)
-  int rs_defer;
-  uint64_t* rs_state;
-  // epoch mode (edb_ag_gemm_epoch_bf16): no handshake with the peers inside the kernel — an
-  // edb_epoch_barrier earlier on the stream made every member's shard final, and the next barrier
-  // comes before anybody overwrites it.  Only the local chunk flags (comm CTAs -> MMA CTAs) remain.
-  int epoch;
   // all-gather PREFETCH riding on a plain GEMM (edb_gemm_pf_bf16): the first pf_ctas CTAs of the
   // grid do no MMA work; they copy, for each item and each group member p, the byte range
   // [src_off, src_off + bytes) of p's symmetric heap into local dst_off + p * dst_stride — the
@@ -384,31 +365,22 @@ struct FusedArgs {
   int64_t pf_sstride[kMaxPfItems];
   int pf_inplace[kMaxPfItems];
 };
-constexpr int F_PUSHED = F_CHUNK + 8;  // [40..47] PUSHED[p]: peer p's deferred-RS tiles of op q landed
 
 struct CMaps {
-  CUtensorMap m[kMaxGroup];  // MODE_RS: store map of member p's receive slot [me]; MODE_AG: m[0] = local shard
+  CUtensorMap m[kMaxGroup];  // push: store map of member p's receive slot [me]; MODE_AG: m[0] = local shard
 };
 
 template <int MODE>
 __device__ __forceinline__ void tile_coords(int t, const GemmParams& p, const FusedArgs& fa,
-                                            int& m_blk, int& n_blk, int& chunk) {
+                                            int& m_blk, int& n_blk) {
   if (MODE == MODE_AG) {
     // n-tiles in rotated order starting at the tile that holds my own shard (needs no transfer),
-    // then in the order the comm CTAs pull the peers' shards
+    // then in the order the comm CTAs pull the peers' shards; a tile may span several shards (see
+    // the producer)
     const int ni = t / p.m_tiles;
     n_blk = (fa.ag_first_tile + ni) % p.n_tiles;
     m_blk = t - ni * p.m_tiles;
-    chunk = -1;  // a tile may span several shards: see the producer
-  } else if (MODE == MODE_RS) {
-    const int mtc = p.m_tiles / fa.f.n;  // m-tiles per chunk
-    const int tpc = mtc * p.n_tiles;
-    const int ci = t / tpc, w = t - ci * tpc;
-    chunk = (fa.f.me + 1 + ci) % fa.f.n;  // own rows last: their reduction needs the peers anyway
-    m_blk = chunk * mtc + w % mtc;
-    n_blk = w / mtc;
   } else {
-    chunk = 0;
     m_blk = (t % p.m_tiles + p.m_rot) % p.m_tiles;
     n_blk = t / p.m_tiles;
   }
@@ -519,12 +491,13 @@ __global__ void __launch_bounds__(32, 1) k_ag_prefetch(const __grid_constant__ F
   pf_role(fa, smem, (int)blockIdx.x, (int)gridDim.x);
 }
 
-// Epoch-mode comm CTA: the same TMA bulk-copy ring, but ONE software pipeline over the blocks of
-// all shards — no drain between shards (the per-op variant below pays a load + store latency per
-// shard, ~4 us x (n-1) at n = 8) and no flag traffic with the peers at all.  A shard is announced
-// to the MMA CTAs once `wait_group` proves its last store complete, which lags kLag stores behind.
-__device__ __forceinline__ void ag_comm_role_epoch(const FusedArgs& fa, uint8_t* smem, int comm_idx,
-                                                   uint64_t q) {
+// MODE_AG comm CTA: one thread drives a TMA bulk-copy ring  peer HBM -> smem -> local HBM, ONE
+// software pipeline over the blocks of all shards — no drain between shards (a drain costs a load +
+// store latency per shard, ~4 us x (n-1) at n = 8) and no flag traffic with the peers at all.  A
+// shard is announced to the MMA CTAs once `wait_group` proves its last store complete, which lags
+// kLag stores behind.
+__device__ __forceinline__ void ag_comm_role(const FusedArgs& fa, uint8_t* smem, int comm_idx,
+                                             uint64_t q) {
   constexpr int S = 8, D = 5, SLOT = 16384, kLag = 2;
   uint64_t* full = reinterpret_cast<uint64_t*>(smem + S * SLOT);
   const FlagCtx& f = fa.f;
@@ -604,151 +577,6 @@ __device__ __forceinline__ void ag_comm_role_epoch(const FusedArgs& fa, uint8_t*
   }
 }
 
-// MODE_AG comm CTA: one thread drives a TMA bulk-copy ring  peer HBM -> smem -> local HBM.
-__device__ __forceinline__ void ag_comm_role(const FusedArgs& fa, uint8_t* smem, int comm_idx,
-                                             uint64_t q) {
-  constexpr int S = 8, D = 4, SLOT = 16384;
-  uint64_t* full = reinterpret_cast<uint64_t*>(smem + S * SLOT);
-  const FlagCtx& f = fa.f;
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < S; ++s) mbar_init(&full[s], 1);
-    fence_barrier_init();
-  }
-  __syncthreads();
-  if (threadIdx.x != 0) return;
-  const int w_chunk = F_CHUNK, w_tile = F_TILECNT;
-  if (comm_idx == 0) {
-    // my shard was written by earlier kernels of this stream: publish it
-    __threadfence_system();
-    for (int pidx = 0; pidx < f.n; ++pidx)
-      if (pidx != f.me) st_release_sys(f.peer[pidx] + F_READY + f.me, q);
-  }
-  uint32_t n_load = 0, n_store = 0;
-  const int64_t per = ((fa.shard_bytes + fa.n_comm - 1) / fa.n_comm + SLOT - 1) / SLOT * SLOT;
-  const int64_t lo = (int64_t)comm_idx * per;
-  const int64_t hi = lo + per < fa.shard_bytes ? lo + per : fa.shard_bytes;
-  const int64_t nblk = hi > lo ? (hi - lo + SLOT - 1) / SLOT : 0;
-  for (int k = 0; k < f.n; ++k) {
-    const int c = (f.me + k) % f.n;
-    if (c != f.me) spin_wait_sys(f.local + F_READY + c, q, f.timeout_ns, f.local + F_ERR);
-    const char* src = fa.shard_src[c] + lo;
-    char* dst = fa.full_dst + (int64_t)c * fa.shard_bytes + lo;
-    for (int64_t i = 0; i < nblk + D; ++i) {
-      if (i < nblk) {
-        const uint32_t slot = n_load % S;
-        if (n_load >= (uint32_t)S) tma_store_wait_read<S - D - 1>();
-        const int64_t left = hi - lo - i * SLOT;
-        const uint32_t bytes = (uint32_t)(left < SLOT ? left : SLOT);
-        mbar_expect_tx(&full[slot], bytes);
-        bulk_load(smem + slot * SLOT, src + i * SLOT, bytes, &full[slot]);
-        ++n_load;
-      }
-      if (i >= D) {
-        const int64_t j = i - D;
-        const uint32_t slot = n_store % S;
-        mbar_wait(&full[slot], (n_store / S) & 1);
-        const int64_t left = hi - lo - j * SLOT;
-        const uint32_t bytes = (uint32_t)(left < SLOT ? left : SLOT);
-        bulk_store(dst + j * SLOT, smem + slot * SLOT, bytes);
-        tma_store_commit();
-        ++n_store;
-      }
-    }
-    tma_store_wait_all();
-    fence_proxy_async_all();
-    __threadfence();
-    const unsigned long long prev =
-        atomicAdd(reinterpret_cast<unsigned long long*>(f.local + w_tile + c), 1ULL);
-    if (prev == (unsigned long long)fa.n_comm - 1) {
-      f.local[w_tile + c] = 0;
-      __threadfence();
-      st_release_gpu(f.local + w_chunk + c, q);
-    }
-  }
-  // end of the op: DONE to the peers, SEQ locally — but only after every CTA of this launch has
-  // read the old SEQ (slow starters would otherwise compute the wrong op number)
-  const unsigned long long prev =
-      atomicAdd(reinterpret_cast<unsigned long long*>(f.local + F_CNT_B), 1ULL);
-  if (prev == (unsigned long long)fa.n_comm - 1) {
-    f.local[F_CNT_B] = 0;
-    while (ld_acquire_gpu(f.local + F_CNT_C) < (uint64_t)gridDim.x) __nanosleep(64);
-    f.local[F_CNT_C] = 0;
-    __threadfence_system();
-    for (int pidx = 0; pidx < f.n; ++pidx)
-      if (pidx != f.me) st_release_sys(f.peer[pidx] + F_DONE + f.me, q);
-    st_release_gpu(f.local + F_SEQ, q);
-  }
-}
-
-template <typename Out>
-__device__ __forceinline__ void rs_store(Out* out, int64_t i, const float* acc) {
-  if (sizeof(Out) == 4) {
-    float4* o = reinterpret_cast<float4*>(out) + 2 * i;
-    o[0] = make_float4(acc[0], acc[1], acc[2], acc[3]);
-    o[1] = make_float4(acc[4], acc[5], acc[6], acc[7]);
-  } else {
-    uint4 o;
-    __nv_bfloat162 h0 = __floats2bfloat162_rn(acc[0], acc[1]);
-    __nv_bfloat162 h1 = __floats2bfloat162_rn(acc[2], acc[3]);
-    __nv_bfloat162 h2 = __floats2bfloat162_rn(acc[4], acc[5]);
-    __nv_bfloat162 h3 = __floats2bfloat162_rn(acc[6], acc[7]);
-    o.x = *reinterpret_cast<uint32_t*>(&h0);
-    o.y = *reinterpret_cast<uint32_t*>(&h1);
-    o.z = *reinterpret_cast<uint32_t*>(&h2);
-    o.w = *reinterpret_cast<uint32_t*>(&h3);
-    reinterpret_cast<uint4*>(out)[i] = o;
-  }
-}
-
-// Sum the n receive slots in rank order (fp32), scale, cast.  All slots are local memory; every
-// load of an iteration is issued before the first add so that n x U 16-byte loads are in flight.
-template <typename Out>
-__device__ __forceinline__ void rs_tail_reduce(const FusedArgs& fa, uint64_t tid, uint64_t nthr) {
-  const int64_t nvec = fa.chunk_bytes / 16;  // 8 bf16 per vector
-  const int n = fa.f.n;
-  Out* out = static_cast<Out*>(fa.rs_dst);
-  constexpr int U = 2;
-  for (int64_t i0 = tid; i0 < nvec; i0 += U * nthr) {
-    uint4 raw[U][kMaxGroup];
-#pragma unroll
-    for (int u = 0; u < U; ++u) {
-      const int64_t i = i0 + u * (int64_t)nthr;
-      if (i < nvec) {
-#pragma unroll
-        for (int s = 0; s < kMaxGroup; ++s)
-          if (s < n)
-            raw[u][s] = *reinterpret_cast<const uint4*>(fa.recv_base + (int64_t)s * fa.chunk_bytes + i * 16);
-      }
-    }
-#pragma unroll
-    for (int u = 0; u < U; ++u) {
-      const int64_t i = i0 + u * (int64_t)nthr;
-      if (i >= nvec) break;
-      float acc[8];
-#pragma unroll
-      for (int s = 0; s < kMaxGroup; ++s) {
-        if (s < n) {
-          const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&raw[u][s]);
-#pragma unroll
-          for (int e = 0; e < 4; ++e) {
-            const float2 v = __bfloat1622float2(h[e]);
-            if (s == 0) {
-              acc[2 * e] = v.x;
-              acc[2 * e + 1] = v.y;
-            } else {
-              acc[2 * e] += v.x;
-              acc[2 * e + 1] += v.y;
-            }
-          }
-        }
-      }
-#pragma unroll
-      for (int e = 0; e < 8; ++e) acc[e] *= fa.rs_scale;
-      rs_store<Out>(out, i, acc);
-    }
-  }
-}
-
 // ---- kernel ------------------------------------------------------------------------------------------
 
 // CL = 2: thread-block cluster of two CTAs = one 256 x BN tile computed with cta_group::2 UMMA.
@@ -768,37 +596,20 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) &
                                              ~static_cast<uintptr_t>(1023));
   __shared__ uint64_t s_q;
-  __shared__ int s_last;
   uint64_t q = 0;
-  const int n_gemm_ctas = (MODE == MODE_AG) ? (int)gridDim.x - fa.n_comm
-                                             : (MODE == MODE_PLAIN ? (int)gridDim.x - fa.pf_ctas : (int)gridDim.x);
+  const int n_gemm_ctas = (int)gridDim.x - (MODE == MODE_AG ? fa.n_comm : fa.pf_ctas);
 
-  if (MODE == MODE_RS) {
-    if (fa.rs_defer) {
-      // no lockstep with the peers: the receive slots belong to this weight alone, and the owners
-      // finished reducing their previous content in op rs_state[1] (same op number on every rank)
-      if (threadIdx.x == 0) s_q = ld_relaxed_gpu(fa.f.local + F_SEQ) + 1;
-      if ((int)threadIdx.x < fa.f.n && (int)threadIdx.x != fa.f.me) {
-        const uint64_t prev = ld_relaxed_gpu(fa.rs_state + 1);
-        if (prev) spin_wait_sys(fa.f.local + F_DONE + threadIdx.x, prev, fa.f.timeout_ns, fa.f.local + F_ERR);
-      }
-      __syncthreads();
-      q = s_q;
-    } else {
-      q = begin_op(fa.f, &s_q);  // WAR guard: peers are done with my buffers of earlier ops
-    }
-  } else if (MODE == MODE_AG) {
+  if (MODE == MODE_AG) {
     if (threadIdx.x == 0) {
-      s_q = ld_relaxed_gpu(fa.f.local + (fa.epoch ? F_AGSEQ : F_SEQ)) + 1;
-      atomicAdd(reinterpret_cast<unsigned long long*>(fa.f.local + (fa.epoch ? F_AGCNT : F_CNT_C)), 1ULL);
+      s_q = ld_relaxed_gpu(fa.f.local + F_AGSEQ) + 1;
+      atomicAdd(reinterpret_cast<unsigned long long*>(fa.f.local + F_AGCNT), 1ULL);
     }
     __syncthreads();
     q = s_q;
     // the comm CTAs are the producers the MMA CTAs spin on: they get the LOWEST block indices so
     // that they are scheduled first even when the grid is not fully co-resident
     if ((int)blockIdx.x < fa.n_comm) {
-      if (fa.epoch) ag_comm_role_epoch(fa, smem, (int)blockIdx.x, q);
-      else ag_comm_role(fa, smem, (int)blockIdx.x, q);
+      ag_comm_role(fa, smem, (int)blockIdx.x, q);
       return;
     }
   }
@@ -807,8 +618,7 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
     pf_role(fa, smem, (int)blockIdx.x, fa.pf_ctas);
     return;
   }
-  const int cta = (MODE == MODE_AG) ? (int)blockIdx.x - fa.n_comm
-                                    : (MODE == MODE_PLAIN ? (int)blockIdx.x - fa.pf_ctas : (int)blockIdx.x);
+  const int cta = (int)blockIdx.x - (MODE == MODE_AG ? fa.n_comm : fa.pf_ctas);
 
   uint8_t* smem_a = smem;
   uint8_t* smem_b = smem + kStages * kSmemABytes;
@@ -871,13 +681,12 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
           kb0 = (u / num_tiles) * p.kb_per_split;
           kb1 = kb0 + p.kb_per_split < k_blocks ? kb0 + p.kb_per_split : k_blocks;
         }
-        int m_blk, n_blk, chunk;
+        int m_blk, n_blk;
         if (CL == 2) {
-          chunk = 0;
           m_blk = 2 * ((t % pm_tiles + p.m_rot) % pm_tiles) + crank;
           n_blk = t / pm_tiles;
         } else {
-          tile_coords<MODE>(t, p, fa, m_blk, n_blk, chunk);
+          tile_coords<MODE>(t, p, fa, m_blk, n_blk);
         }
         const CUtensorMap* bmap = &tmap_b;
         int b_row = n_blk * BN;
@@ -888,7 +697,7 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
             b_row = n_blk * BN - fa.f.me * fa.ag_rows;
           } else if (n_blk != ready_chunk) {
             for (int c = c_lo; c <= c_hi; ++c)
-              spin_wait_gpu(fa.f.local + (fa.epoch ? F_AGCHUNK : F_CHUNK) + c, q);
+              spin_wait_gpu(fa.f.local + F_AGCHUNK + c, q);
             fence_proxy_async_all();
             ready_chunk = n_blk;
           }
@@ -1009,13 +818,12 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
     int ebuf = 0;
     for (int u = unit0; u < num_units; u += unit_stride) {
       const int t = (MODE == MODE_PLAIN) ? u % num_tiles : u;
-      int m_blk, n_blk, chunk;
+      int m_blk, n_blk;
       if (CL == 2) {
-        chunk = 0;
         m_blk = 2 * ((t % pm_tiles + p.m_rot) % pm_tiles) + crank;
         n_blk = t / pm_tiles;
       } else {
-        tile_coords<MODE>(t, p, fa, m_blk, n_blk, chunk);
+        tile_coords<MODE>(t, p, fa, m_blk, n_blk);
       }
       if (MODE == MODE_PLAIN && p.splits > 1) {
         // split-K: this unit's fp32 partial goes straight from registers to the workspace (one
@@ -1058,10 +866,6 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
       }
       const CUtensorMap* cmap = &tmap_c;
       int c_row = m_blk * BM;
-      if (MODE == MODE_RS) {
-        cmap = &cm.m[chunk];  // receive slot [me] of the rank that owns these rows
-        c_row = (m_blk - chunk * (p.m_tiles / fa.f.n)) * BM;
-      }
       if (MODE == MODE_PLAIN && p.push_n > 0) {
         const int owner = m_blk / p.push_mtc;
         cmap = &cm.m[owner];
@@ -1172,20 +976,6 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
         }
         ebuf ^= 1;
       }
-      if (MODE == MODE_RS && issuer) {
-        // this tile now sits (or is in flight to) its owner: count it, and when the last tile of
-        // the chunk has landed tell the owner that source `me` is complete
-        tma_store_wait_all();
-        fence_proxy_async_all();
-        __threadfence_system();
-        const unsigned long long prev = atomicAdd(
-            reinterpret_cast<unsigned long long*>(fa.f.local + F_TILECNT + chunk), 1ULL);
-        if (prev == (unsigned long long)fa.tiles_per_chunk - 1) {
-          fa.f.local[F_TILECNT + chunk] = 0;
-          __threadfence_system();
-          st_release_sys(fa.f.peer[chunk] + (fa.rs_defer ? F_PUSHED : F_CHUNK) + fa.f.me, q);
-        }
-      }
       if (++as == 2) {
         as = 0;
         aphase ^= 1;
@@ -1214,38 +1004,41 @@ __global__ void __launch_bounds__(kGemmThreads, 1)
     if (CL == 2) tmem_dealloc_2cta(tmem_base, Cfg::kTmemCols);
     else tmem_dealloc(tmem_base, Cfg::kTmemCols);
   }
-
-  if (MODE == MODE_RS) {
-    if (fa.rs_defer) {
-      if (blockIdx.x == 0 && threadIdx.x == 0) fa.rs_state[0] = q;  // read by k_rs_finish (later kernel)
-    } else {
-      // ===== tail: reduce my rows from the n receive slots (all local), rank order =====
-      if (threadIdx.x < fa.f.n)
-        spin_wait_sys(fa.f.local + F_CHUNK + threadIdx.x, q, fa.f.timeout_ns, fa.f.local + F_ERR);
-      __syncthreads();
-      const uint64_t tid = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-      const uint64_t nthr = (uint64_t)gridDim.x * blockDim.x;
-      if (fa.rs_out_dtype == EDB_F32) rs_tail_reduce<float>(fa, tid, nthr);
-      else rs_tail_reduce<__nv_bfloat16>(fa, tid, nthr);
-    }
-    finish_op(fa.f, q, &s_last, gridDim.x);
-  }
 }
 
 // ---- deferred reduce-scatter: reduce the receive slots of many pushed GEMMs in one launch -----------
+// An edb_epoch_barrier earlier on the stream made every slot complete: purely local memory traffic.
 constexpr int kRsMaxItems = 160;
 constexpr int kRsFinishThreads = 256;
 constexpr int64_t kRsFinishChunkVecs = 4096;  // 64 KiB of bf16 per slot and work unit
+
+template <typename Out>
+__device__ __forceinline__ void rs_store(Out* out, int64_t i, const float* acc) {
+  if (sizeof(Out) == 4) {
+    float4* o = reinterpret_cast<float4*>(out) + 2 * i;
+    o[0] = make_float4(acc[0], acc[1], acc[2], acc[3]);
+    o[1] = make_float4(acc[4], acc[5], acc[6], acc[7]);
+  } else {
+    uint4 o;
+    __nv_bfloat162 h0 = __floats2bfloat162_rn(acc[0], acc[1]);
+    __nv_bfloat162 h1 = __floats2bfloat162_rn(acc[2], acc[3]);
+    __nv_bfloat162 h2 = __floats2bfloat162_rn(acc[4], acc[5]);
+    __nv_bfloat162 h3 = __floats2bfloat162_rn(acc[6], acc[7]);
+    o.x = *reinterpret_cast<uint32_t*>(&h0);
+    o.y = *reinterpret_cast<uint32_t*>(&h1);
+    o.z = *reinterpret_cast<uint32_t*>(&h2);
+    o.w = *reinterpret_cast<uint32_t*>(&h3);
+    reinterpret_cast<uint4*>(out)[i] = o;
+  }
+}
 
 struct RsFinishItem {
   const char* recv;     // n slots of chunk_bytes (local)
   void* dst;            // [chunk_bytes / 2] elements of out_dtype
   int64_t chunk_bytes;
-  uint64_t* state;      // [0] op number of the push, [1] op number of this reduction
 };
 struct RsFinishDesc {
-  FlagCtx f;
-  int local_only;  // epoch mode: an edb_epoch_barrier earlier on the stream replaced every handshake
+  int n;  // group size = number of slots
   int n_items;
   float scale;
   int out_dtype;
@@ -1259,31 +1052,8 @@ struct RsFinishDesc {
 template <int NSRC>
 __global__ void __launch_bounds__(kRsFinishThreads, 4)
     k_rs_finish(const __grid_constant__ RsFinishDesc d) {
-  __shared__ uint64_t s_q;
-  __shared__ unsigned long long s_need;
-  __shared__ int s_last;
-  if (threadIdx.x == 0) {
-    s_q = ld_relaxed_gpu(d.f.local + F_SEQ) + 1;
-    s_need = 0;
-  }
-  __syncthreads();
-  if (!d.local_only) {
-    // every source must have landed its tiles of the latest push among the items (flags are
-    // monotonic and a source's pushes complete in stream order, so the latest covers the earlier)
-    unsigned long long need = 0;
-    for (int i = threadIdx.x; i < d.n_items; i += blockDim.x) {
-      const unsigned long long e = ld_relaxed_gpu(d.it[i].state);
-      need = e > need ? e : need;
-    }
-    if (need) atomicMax(&s_need, need);
-    __syncthreads();
-    if ((int)threadIdx.x < d.f.n)
-      spin_wait_sys(d.f.local + F_PUSHED + threadIdx.x, s_need, d.f.timeout_ns, d.f.local + F_ERR);
-    __syncthreads();
-  }
-  const uint64_t q = s_q;
   const int total_units = d.first_unit[d.n_items];
-  const int n = NSRC > 0 ? NSRC : d.f.n;
+  const int n = NSRC > 0 ? NSRC : d.n;
   constexpr int MAXS = NSRC > 0 ? NSRC : kMaxGroup;
   constexpr int U = NSRC > 0 ? (8 / NSRC > 0 ? 8 / NSRC : 1) : 1;
   for (int u = blockIdx.x; u < total_units; u += gridDim.x) {
@@ -1340,11 +1110,6 @@ __global__ void __launch_bounds__(kRsFinishThreads, 4)
       }
     }
   }
-  if (d.local_only) return;
-  // remember which op reduced these slots (the next pushes check the owners' DONE against it)
-  if (blockIdx.x == 0)
-    for (int i = threadIdx.x; i < d.n_items; i += blockDim.x) d.it[i].state[1] = q;
-  finish_op(d.f, q, &s_last, gridDim.x);
 }
 
 // push mode: row r of C belongs to member r / rows_per and goes to base[owner] + (r % rows_per) * ldc
@@ -1475,29 +1240,28 @@ static int launch_gemm_cl(const CUtensorMap& ta, const CUtensorMap& tb, const CU
   return cuda_check(cudaGetLastError(), "k_gemm_bf16 launch");
 }
 
-template <int BN, bool AK, bool BK_, int MODE>
-static int launch_gemm(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tc,
-                       const GemmParams& p, const FusedArgs& fa, const CMaps& cm, int grid,
-                       cudaStream_t st, int cl = 1) {
-  if (MODE == MODE_PLAIN && cl == 2)
-    return launch_gemm_cl<BN, AK, BK_, MODE_PLAIN, 2>(ta, tb, tc, p, fa, cm, grid, st);
-  return launch_gemm_cl<BN, AK, BK_, MODE, 1>(ta, tb, tc, p, fa, cm, grid, st);
+template <int BN, bool AK, bool BK_>
+static int launch_gemm_plain(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tc,
+                             const GemmParams& p, const FusedArgs& fa, const CMaps& cm, int grid,
+                             cudaStream_t st, int cl) {
+  if (cl == 2) return launch_gemm_cl<BN, AK, BK_, MODE_PLAIN, 2>(ta, tb, tc, p, fa, cm, grid, st);
+  return launch_gemm_cl<BN, AK, BK_, MODE_PLAIN, 1>(ta, tb, tc, p, fa, cm, grid, st);
 }
 
-template <int MODE>
-static int dispatch_gemm(int bn, bool a_k, bool b_k, const CUtensorMap& ta, const CUtensorMap& tb,
-                         const CUtensorMap& tc, const GemmParams& p, const FusedArgs& fa,
-                         const CMaps& cm, int grid, cudaStream_t st, int cl = 1) {
+static int dispatch_gemm_plain(int bn, bool a_k, bool b_k, const CUtensorMap& ta,
+                               const CUtensorMap& tb, const CUtensorMap& tc, const GemmParams& p,
+                               const FusedArgs& fa, const CMaps& cm, int grid, cudaStream_t st,
+                               int cl) {
   const int key = (bn == 256 ? 4 : 0) | (a_k ? 2 : 0) | (b_k ? 1 : 0);
   switch (key) {
-    case 7: return launch_gemm<256, true, true, MODE>(ta, tb, tc, p, fa, cm, grid, st, cl);
-    case 6: return launch_gemm<256, true, false, MODE>(ta, tb, tc, p, fa, cm, grid, st, cl);
-    case 5: return launch_gemm<256, false, true, MODE>(ta, tb, tc, p, fa, cm, grid, st, cl);
-    case 4: return launch_gemm<256, false, false, MODE>(ta, tb, tc, p, fa, cm, grid, st, cl);
-    case 3: return launch_gemm<128, true, true, MODE>(ta, tb, tc, p, fa, cm, grid, st, cl);
-    case 2: return launch_gemm<128, true, false, MODE>(ta, tb, tc, p, fa, cm, grid, st, cl);
-    case 1: return launch_gemm<128, false, true, MODE>(ta, tb, tc, p, fa, cm, grid, st, cl);
-    default: return launch_gemm<128, false, false, MODE>(ta, tb, tc, p, fa, cm, grid, st, cl);
+    case 7: return launch_gemm_plain<256, true, true>(ta, tb, tc, p, fa, cm, grid, st, cl);
+    case 6: return launch_gemm_plain<256, true, false>(ta, tb, tc, p, fa, cm, grid, st, cl);
+    case 5: return launch_gemm_plain<256, false, true>(ta, tb, tc, p, fa, cm, grid, st, cl);
+    case 4: return launch_gemm_plain<256, false, false>(ta, tb, tc, p, fa, cm, grid, st, cl);
+    case 3: return launch_gemm_plain<128, true, true>(ta, tb, tc, p, fa, cm, grid, st, cl);
+    case 2: return launch_gemm_plain<128, true, false>(ta, tb, tc, p, fa, cm, grid, st, cl);
+    case 1: return launch_gemm_plain<128, false, true>(ta, tb, tc, p, fa, cm, grid, st, cl);
+    default: return launch_gemm_plain<128, false, false>(ta, tb, tc, p, fa, cm, grid, st, cl);
   }
 }
 
@@ -1755,7 +1519,7 @@ static int gemm_plain_impl(void* C, const void* A, const void* B, const void* bi
     grid = tiles < sms_gemm ? tiles : sms_gemm;
   }
   grid += fa.pf_ctas;
-  rc = dispatch_gemm<MODE_PLAIN>(bn, a_kmajor != 0, b_kmajor != 0, ta, tb, tc, p, fa, cm, grid, st, cl);
+  rc = dispatch_gemm_plain(bn, a_kmajor != 0, b_kmajor != 0, ta, tb, tc, p, fa, cm, grid, st, cl);
   if (rc || p.splits == 1) return rc;
   const int64_t groups = (int64_t)M * (p.ldp / 4);
   int rgrid = (int)((groups + 255) / 256);
@@ -1850,35 +1614,34 @@ int edb_gemm_push_bf16(int gid, uint64_t recv_off, const void* A, const void* B,
                          &ps);
 }
 
-static int ag_gemm_impl(int gid, void* C, const void* A, const void* bias, uint64_t b_shard_off,
-                        uint64_t b_full_off, int64_t M, int64_t N, int64_t K, int64_t lda,
-                        int64_t ldc, void* stream, int epoch) {
+int edb_ag_gemm_epoch_bf16(int gid, void* C, const void* A, const void* bias, uint64_t b_shard_off,
+                           uint64_t b_full_off, int64_t M, int64_t N, int64_t K, int64_t lda,
+                           int64_t ldc, void* stream) {
   FusedArgs fa;
   memset(&fa, 0, sizeof(fa));
-  fa.epoch = epoch;
   int rc = fill_flagctx(&fa.f, gid);
   if (rc) return rc;
   Runtime& r = rt();
   const Group& g = r.groups[gid];
   const int n = g.n, me = g.me;
-  if (N % n) return set_error(EDB_E_UNSUPPORTED, "edb_ag_gemm_bf16: N %% group size != 0");
+  if (N % n) return set_error(EDB_E_UNSUPPORTED, "edb_ag_gemm_epoch_bf16: N %% group size != 0");
   const int64_t rows = N / n;
   int bn = 0;
   if (N % 256 == 0) bn = 256;
   else if (N % 128 == 0) bn = 128;
-  else return set_error(EDB_E_UNSUPPORTED, "edb_ag_gemm_bf16: N=%lld not a multiple of 128",
+  else return set_error(EDB_E_UNSUPPORTED, "edb_ag_gemm_epoch_bf16: N=%lld not a multiple of 128",
                         (long long)N);
   if (rows % 8)
-    return set_error(EDB_E_UNSUPPORTED, "edb_ag_gemm_bf16: shard rows %lld not a multiple of 8",
+    return set_error(EDB_E_UNSUPPORTED, "edb_ag_gemm_epoch_bf16: shard rows %lld not a multiple of 8",
                      (long long)rows);
-  if (K & 7) return set_error(EDB_E_UNSUPPORTED, "edb_ag_gemm_bf16: K must be a multiple of 8");
+  if (K & 7) return set_error(EDB_E_UNSUPPORTED, "edb_ag_gemm_epoch_bf16: K must be a multiple of 8");
   const size_t shard_bytes = (size_t)rows * K * 2;
   if (b_shard_off < kUserOffset || b_shard_off + shard_bytes > r.heap_bytes || (b_shard_off & 15) ||
       b_full_off < kUserOffset || b_full_off + shard_bytes * n > r.heap_bytes || (b_full_off & 1023))
-    return set_error(EDB_E_INVALID, "edb_ag_gemm_bf16: bad symmetric offsets");
+    return set_error(EDB_E_INVALID, "edb_ag_gemm_epoch_bf16: bad symmetric offsets");
   const char* shard = r.heap + b_shard_off;
   char* full = r.heap + b_full_off;
-  rc = check_operands(A, full, C, bias, M, N, K, lda, K, ldc, "edb_ag_gemm_bf16");
+  rc = check_operands(A, full, C, bias, M, N, K, lda, K, ldc, "edb_ag_gemm_epoch_bf16");
   if (rc) return rc;
   CUtensorMap ta, tb, tc;
   rc = make_tmap(&ta, A, K, M, lda, BK, BM);
@@ -1926,77 +1689,28 @@ static int ag_gemm_impl(int gid, void* C, const void* A, const void* bias, uint6
   const int tiles = p.m_tiles * p.n_tiles;
   int gemm_ctas = sms - n_comm;
   if (gemm_ctas > tiles) gemm_ctas = tiles;
-  return dispatch_gemm<MODE_AG>(bn, true, true, ta, tb, tc, p, fa, cm, gemm_ctas + n_comm,
-                                (cudaStream_t)stream);
-}
-
-int edb_ag_gemm_bf16(int gid, void* C, const void* A, const void* bias, uint64_t b_shard_off,
-                     uint64_t b_full_off, int64_t M, int64_t N, int64_t K, int64_t lda, int64_t ldc,
-                     void* stream) {
-  return ag_gemm_impl(gid, C, A, bias, b_shard_off, b_full_off, M, N, K, lda, ldc, stream, 0);
-}
-
-int edb_ag_gemm_epoch_bf16(int gid, void* C, const void* A, const void* bias, uint64_t b_shard_off,
-                           uint64_t b_full_off, int64_t M, int64_t N, int64_t K, int64_t lda,
-                           int64_t ldc, void* stream) {
-  return ag_gemm_impl(gid, C, A, bias, b_shard_off, b_full_off, M, N, K, lda, ldc, stream, 1);
-}
-
-static int gemm_rs_impl(int gid, void* dst, uint64_t recv_off, uint64_t state_off, bool defer,
-                        const void* A, const void* B, int64_t M, int64_t N, int64_t K, int64_t lda,
-                        int64_t ldb, int a_kmajor, int b_kmajor, float post_scale, int out_dtype,
-                        void* stream);
-
-int edb_gemm_rs_bf16(int gid, void* dst, uint64_t recv_off, const void* A, const void* B,
-                     int64_t M, int64_t N, int64_t K, int64_t lda, int64_t ldb, int a_kmajor,
-                     int b_kmajor, float post_scale, int out_dtype, void* stream) {
-  return gemm_rs_impl(gid, dst, recv_off, 0, false, A, B, M, N, K, lda, ldb, a_kmajor, b_kmajor,
-                      post_scale, out_dtype, stream);
-}
-
-int edb_gemm_rs_push_bf16(int gid, uint64_t recv_off, uint64_t state_off, const void* A,
-                          const void* B, int64_t M, int64_t N, int64_t K, int64_t lda, int64_t ldb,
-                          int a_kmajor, int b_kmajor, void* stream) {
-  Runtime& r = rt();
-  if (!r.inited) return set_error(EDB_E_STATE, "runtime not initialised (call edb_init)");
-  if (state_off < kUserOffset || state_off + 16 > r.heap_bytes || (state_off & 15))
-    return set_error(EDB_E_INVALID, "edb_gemm_rs_push_bf16: bad state offset");
-  return gemm_rs_impl(gid, nullptr, recv_off, state_off, true, A, B, M, N, K, lda, ldb, a_kmajor,
-                      b_kmajor, 1.0f, EDB_BF16, stream);
-}
-
-static int rs_finish_impl(int gid, int n_items, void* const* dsts, const uint64_t* recv_offs,
-                          const uint64_t* state_offs, const int64_t* chunk_bytes, float post_scale,
-                          int out_dtype, void* stream, int local_only);
-
-int edb_rs_finish(int gid, int n_items, void* const* dsts, const uint64_t* recv_offs,
-                  const uint64_t* state_offs, const int64_t* chunk_bytes, float post_scale,
-                  int out_dtype, void* stream) {
-  return rs_finish_impl(gid, n_items, dsts, recv_offs, state_offs, chunk_bytes, post_scale,
-                        out_dtype, stream, 0);
+  // A and B are K-major (C = A.Bᵀ, nn.Linear fwd): the only layout this kernel is built for
+  if (bn == 256)
+    return launch_gemm_cl<256, true, true, MODE_AG, 1>(ta, tb, tc, p, fa, cm, gemm_ctas + n_comm,
+                                                       (cudaStream_t)stream);
+  return launch_gemm_cl<128, true, true, MODE_AG, 1>(ta, tb, tc, p, fa, cm, gemm_ctas + n_comm,
+                                                     (cudaStream_t)stream);
 }
 
 int edb_rs_finish_local(int gid, int n_items, void* const* dsts, const uint64_t* recv_offs,
                         const int64_t* chunk_bytes, float post_scale, int out_dtype, void* stream) {
-  return rs_finish_impl(gid, n_items, dsts, recv_offs, nullptr, chunk_bytes, post_scale, out_dtype,
-                        stream, 1);
-}
-
-static int rs_finish_impl(int gid, int n_items, void* const* dsts, const uint64_t* recv_offs,
-                          const uint64_t* state_offs, const int64_t* chunk_bytes, float post_scale,
-                          int out_dtype, void* stream, int local_only) {
   if (n_items <= 0) return EDB_OK;
   if (out_dtype != EDB_BF16 && out_dtype != EDB_F32)
-    return set_error(EDB_E_UNSUPPORTED, "edb_rs_finish: out dtype must be bf16 or f32");
+    return set_error(EDB_E_UNSUPPORTED, "edb_rs_finish_local: out dtype must be bf16 or f32");
   Runtime& r = rt();
+  if (!r.inited) return set_error(EDB_E_STATE, "runtime not initialised (call edb_init)");
+  if (gid < 0 || gid >= r.ngroups) return set_error(EDB_E_INVALID, "bad group id %d", gid);
+  const int n = r.groups[gid].n;
   cudaStream_t st = (cudaStream_t)stream;
   int done = 0;
   while (done < n_items) {
     RsFinishDesc d;
-    int rc = fill_flagctx(&d.f, gid);
-    if (rc) return rc;
-    const int n = d.f.n;
-    d.local_only = local_only;
+    d.n = n;
     d.scale = post_scale;
     d.out_dtype = out_dtype;
     d.first_unit[0] = 0;
@@ -2005,18 +1719,15 @@ static int rs_finish_impl(int gid, int n_items, void* const* dsts, const uint64_
     for (; done < n_items && k < kRsMaxItems; ++done, ++k) {
       const int64_t cb = chunk_bytes[done];
       if (cb <= 0 || (cb & 15) || ((uintptr_t)dsts[done] & 15))
-        return set_error(EDB_E_INVALID, "edb_rs_finish: item %d: chunk bytes / dst alignment", done);
+        return set_error(EDB_E_INVALID, "edb_rs_finish_local: item %d: chunk bytes / dst alignment", done);
       if (recv_offs[done] < kUserOffset || recv_offs[done] + (uint64_t)cb * n > r.heap_bytes ||
-          (recv_offs[done] & 15) ||
-          (!local_only && (state_offs[done] < kUserOffset || state_offs[done] + 16 > r.heap_bytes ||
-                           (state_offs[done] & 15))))
-        return set_error(EDB_E_INVALID, "edb_rs_finish: item %d: bad symmetric offset", done);
+          (recv_offs[done] & 15))
+        return set_error(EDB_E_INVALID, "edb_rs_finish_local: item %d: bad symmetric offset", done);
       d.it[k].recv = r.heap + recv_offs[done];
       d.it[k].dst = dsts[done];
       d.it[k].chunk_bytes = cb;
-      d.it[k].state = local_only ? nullptr : reinterpret_cast<uint64_t*>(r.heap + state_offs[done]);
       units += (cb / 16 + kRsFinishChunkVecs - 1) / kRsFinishChunkVecs;
-      if (units > 0x7fffffffLL) return set_error(EDB_E_UNSUPPORTED, "edb_rs_finish: too much work");
+      if (units > 0x7fffffffLL) return set_error(EDB_E_UNSUPPORTED, "edb_rs_finish_local: too much work");
       d.first_unit[k + 1] = (int)units;
     }
     d.n_items = k;
@@ -2028,88 +1739,10 @@ static int rs_finish_impl(int gid, int n_items, void* const* dsts, const uint64_
       default: k_rs_finish<0><<<grid, kRsFinishThreads, 0, st>>>(d); break;
     }
     count_launch();
-    rc = cuda_check(cudaGetLastError(), "k_rs_finish launch");
+    const int rc = cuda_check(cudaGetLastError(), "k_rs_finish launch");
     if (rc) return rc;
   }
   return EDB_OK;
-}
-
-static int gemm_rs_impl(int gid, void* dst, uint64_t recv_off, uint64_t state_off, bool defer,
-                        const void* A, const void* B, int64_t M, int64_t N, int64_t K, int64_t lda,
-                        int64_t ldb, int a_kmajor, int b_kmajor, float post_scale, int out_dtype,
-                        void* stream) {
-  FusedArgs fa;
-  memset(&fa, 0, sizeof(fa));
-  int rc = fill_flagctx(&fa.f, gid);
-  if (rc) return rc;
-  Runtime& r = rt();
-  const Group& g = r.groups[gid];
-  const int n = g.n, me = g.me;
-  if (M % n || (M / n) % BM)
-    return set_error(EDB_E_UNSUPPORTED, "edb_gemm_rs_bf16: rows per rank must be a multiple of 128");
-  if (N & 7) return set_error(EDB_E_UNSUPPORTED, "edb_gemm_rs_bf16: N must be a multiple of 8");
-  if (out_dtype != EDB_BF16 && out_dtype != EDB_F32)
-    return set_error(EDB_E_UNSUPPORTED, "edb_gemm_rs_bf16: out dtype must be bf16 or f32");
-  const int64_t rows = M / n;
-  const size_t chunk_bytes = (size_t)rows * N * 2;
-  if (recv_off < kUserOffset || recv_off + chunk_bytes * n > r.heap_bytes || (recv_off & 1023))
-    return set_error(EDB_E_INVALID, "edb_gemm_rs_bf16: bad symmetric offset");
-  char* recv = r.heap + recv_off;
-  rc = check_operands(A, B, recv, nullptr, M, N, K, lda, ldb, N, "edb_gemm_rs_bf16");
-  if (rc) return rc;
-  const int sms = r.sm_count;
-  const int bn = pick_bn(M, N, sms);
-  CUtensorMap ta, tb, tc;
-  if (a_kmajor) rc = make_tmap(&ta, A, K, M, lda, BK, BM);
-  else rc = make_tmap(&ta, A, M, K, lda, 64, BK);
-  if (rc) return rc;
-  if (b_kmajor) rc = make_tmap(&tb, B, K, N, ldb, BK, bn);
-  else rc = make_tmap(&tb, B, N, K, ldb, 64, BK);
-  if (rc) return rc;
-  CMaps cm;
-  memset(&cm, 0, sizeof(cm));
-  for (int pidx = 0; pidx < n; ++pidx) {
-    // rows owned by member pidx land in ITS receive buffer, slot [me]
-    char* slot = r.peer_heap[g.ranks[pidx]] + recv_off + (size_t)me * chunk_bytes;
-    rc = make_tmap(&cm.m[pidx], slot, N, rows, N, 64, BM);
-    if (rc) return rc;
-  }
-  tc = cm.m[me];
-  GemmParams p;
-  p.C = reinterpret_cast<__nv_bfloat16*>(recv);
-  p.bias = nullptr;
-  p.ldc = N;
-  p.M = (int)M;
-  p.N = (int)N;
-  p.K = (int)K;
-  p.m_tiles = (int)(M / BM);
-  p.n_tiles = (int)((N + bn - 1) / bn);
-  p.splits = 1;
-  p.kb_per_split = 0;
-  p.partial = nullptr;
-  p.ldp = 0;
-  p.push_n = 0;
-  p.push_mtc = 1;
-  p.m_rot = 0;
-  p.push_sync = 0;
-  p.aux = nullptr;
-  p.ld_aux = 0;
-  p.epi_op = EPI_NONE;
-  fa.recv_base = recv;
-  fa.chunk_bytes = (int64_t)chunk_bytes;
-  fa.rs_dst = dst;
-  fa.rs_scale = post_scale;
-  fa.rs_out_dtype = out_dtype;
-  fa.tiles_per_chunk = (p.m_tiles / n) * p.n_tiles;
-  fa.rs_defer = defer ? 1 : 0;
-  fa.rs_state = defer ? reinterpret_cast<uint64_t*>(r.heap + state_off) : nullptr;
-  // fused tail: always a full grid — CTAs without a tile still take part in the tail reduction,
-  // which is latency-bound when only a few CTAs read the receive slots (small weight gradients);
-  // push-only: one CTA per tile
-  const int tiles = p.m_tiles * p.n_tiles;
-  const int grid = defer ? (tiles < sms ? tiles : sms) : sms;
-  return dispatch_gemm<MODE_RS>(bn, a_kmajor != 0, b_kmajor != 0, ta, tb, tc, p, fa, cm, grid,
-                                (cudaStream_t)stream);
 }
 
 }  // extern "C"

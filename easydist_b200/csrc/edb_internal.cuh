@@ -43,13 +43,12 @@ enum FlagWord : int {
   F_LLSEQ = 29,   // sequence number of the low-latency ops of this group
   F_CNT_LL = 30,  // last-block counter of the LL kernels
   F_ERRHOST = 31, // device pointer of the pinned host error record (written once at edb_init)
-  F_CHUNK = 32,   // [32..47] per-chunk flags for fused kernels (written by peers / local CTAs)
-  // ---- epoch protocol (edb_epoch_barrier + the *_epoch fused kernels) -------------------------
+  // ---- epoch protocol (edb_epoch_barrier + the fused / push kernels) --------------------------
   // One group-wide barrier per phase of the step instead of a handshake per op: between two
   // barriers peers may read this rank's symmetric operands / write its receive slots freely.
   F_EPOCH = 48,      // [48..55] ARRIVED[p]: member p reached barrier number e   (written by p)
   F_EPOCH_SEQ = 56,  // barriers completed locally                                 (written by me)
-  F_AGSEQ = 57,      // launch number of the epoch-mode AG+GEMM kernels (local chunk-flag epochs)
+  F_AGSEQ = 57,      // launch number of the AG+GEMM kernels (local chunk-flag epochs)
   F_AGCNT = 58,      // CTAs of the current AG+GEMM launch that have read F_AGSEQ
   F_AGDONE = 59,     // comm CTAs of the current launch that have finished
   F_AGCHUNK = 64,    // [64..71] local: peer shard c is in the gathered buffer (launch number)

@@ -189,11 +189,6 @@ __global__ void __launch_bounds__(kThreads) k_push(const __grid_constant__ Gathe
   }
 }
 
-__global__ void __launch_bounds__(32) k_guard(const __grid_constant__ FlagCtx f) {
-  __shared__ uint64_t s_q;
-  begin_op(f, &s_q);
-}
-
 __global__ void __launch_bounds__(32) k_epoch_barrier(const __grid_constant__ FlagCtx f) {
   __shared__ uint64_t s_e;
   epoch_barrier_cta(f, &s_e);
@@ -1247,16 +1242,6 @@ int edb_epoch_barrier(int gid, void* stream) {
   k_epoch_barrier<<<1, 32, 0, (cudaStream_t)stream>>>(f);
   count_launch();
   return cuda_check(cudaGetLastError(), "k_epoch_barrier launch");
-}
-
-int edb_symm_guard(int gid, void* stream) {
-  FlagCtx f;
-  int rc = fill_flagctx(&f, gid);
-  if (rc) return rc;
-  if (f.n <= 1) return EDB_OK;
-  k_guard<<<1, 32, 0, (cudaStream_t)stream>>>(f);
-  count_launch();
-  return cuda_check(cudaGetLastError(), "k_guard launch");
 }
 
 }  // extern "C"

@@ -1504,10 +1504,15 @@ def fuse_collective_gemms(gm, io, rt, ranks, ops=_default_ops, my_index=None):
     """Peephole fusion of reshard edges into the adjacent GEMM (B200 runtime only):
 
       all_gather(param shard) -> view -> t -> mm/addmm        ==>  ops.ag_mm   (AG + GEMM, one kernel)
-      mm -> flatten -> reduce_scatter(avg, dim 0)              ==>  ops.mm_rs   (GEMM + RS, one kernel)
+      mm -> flatten -> reduce_scatter(avg, dim 0)              ==>  ops.mm_push (GEMM pushes its rows
+                                                                   to their owners) + ops.rs_finish
 
-    Returns {placeholder name: SymmBuffer} for parameter shards that must live in the symmetric
-    heap (peers read them directly), after inserting a symm_guard in front of the optimizer."""
+    Epoch protocol: no handshake inside the fused kernels; ONE group barrier in front of the
+    optimizer (all gradient tiles have landed in their owners' slots, nobody still reads the old
+    parameter shards) and ONE behind it (the new shards are final, the slots are free again).
+    Returns ({placeholder name: SymmBuffer} for parameter shards that must live in the symmetric
+    heap (peers read them directly), {"ag_mm", "ag_pf", "mm_rs": number of rewrites}); "mm_rs"
+    counts the GEMM + reduce-scatter pairs turned into pushes."""
     import os
     graph = gm.graph
     n = len(ranks)
@@ -1517,13 +1522,8 @@ def fuse_collective_gemms(gm, io, rt, ranks, ops=_default_ops, my_index=None):
     rehomed = {}
     n_ag = n_rs = 0
     bf16 = torch.bfloat16
-    # epoch protocol (default): no handshake inside the fused kernels; ONE group barrier in front
-    # of the optimizer (all gradient tiles have landed in their owners' slots, nobody still reads the
-    # old parameter shards) and ONE behind it (the new shards are final, the slots are free again).
-    # EDB_EPOCH=0 keeps the per-op flag protocol of the fused kernels.
-    epoch = os.environ.get("EDB_EPOCH", "1") == "1" and hasattr(ops, "epoch_barrier")
     n_pf = 0
-    if epoch and os.environ.get("EDB_AG_PREFETCH", "1") == "1" and hasattr(ops, "gathered"):
+    if os.environ.get("EDB_AG_PREFETCH", "1") == "1":
         # all parameter gathers as prefetches riding on earlier GEMMs (no AG left to fuse below)
         rehomed, n_pf = prefetch_param_gathers(gm, io, rt, ranks, ops, my_index=my_index)
         order = {nd: i for i, nd in enumerate(graph.nodes)}
@@ -1566,11 +1566,8 @@ def fuse_collective_gemms(gm, io, rt, ranks, ops=_default_ops, my_index=None):
         full = rt.alloc(n_out * k_in * 2, align=1024)
         rehomed[ph.name] = shard
         with graph.inserting_before(first):
-            ag_kw = {"_buf": (shard.offset, full.offset)}
-            if epoch:
-                ag_kw["_epoch"] = 1
             fused = graph.call_function(ops.ag_mm, args=(x, ph, list(ranks), n_out, k_in, bias),
-                                        kwargs=ag_kw)
+                                        kwargs={"_buf": (shard.offset, full.offset), "_epoch": 1})
             out = graph.call_function(operator.getitem, args=(fused, 0))
             wfull = graph.call_function(operator.getitem, args=(fused, 1))
             t_new = graph.call_function(aten.t.default, args=(wfull,))
@@ -1582,10 +1579,9 @@ def fuse_collective_gemms(gm, io, rt, ranks, ops=_default_ops, my_index=None):
         n_ag += 1
 
     # ---- GEMM + reduce-scatter -------------------------------------------------------------
-    # deferred form (EDB_DEFER_RS=1): the GEMM only pushes its tiles to the owners; one rs_finish
-    # node in front of the first consumer reduces every weight gradient's slots in a single kernel
-    defer = epoch or (os.environ.get("EDB_DEFER_RS", "0") == "1" and hasattr(ops, "mm_rs_push"))
-    pushed = []  # (token node, recv buffer, state buffer, shard numel, rs_end node)
+    # the GEMM only pushes its tiles to the owners; one rs_finish node in front of the first
+    # consumer reduces every weight gradient's slots in a single kernel
+    pushed = []  # (token node, recv buffer, shard numel, rs_end node)
     for rs_s in [x for x in graph.nodes if x.op == "call_function" and x.target is ops.reduce_scatter_start]:
         f = rs_s.args[0]
         if rs_s.args[1] != "avg" or rs_s.args[2] != 0 or rs_s.kwargs:
@@ -1625,32 +1621,13 @@ def fuse_collective_gemms(gm, io, rt, ranks, ops=_default_ops, my_index=None):
                     nd.meta["val"] = src.t()
             else:
                 a, b = a0, b0
-            if epoch:
-                tok = graph.call_function(ops.mm_push, args=(a, b, list(ranks)),
-                                          kwargs={"_buf": (recv.offset,)})
-                pushed.append((tok, recv, None, M // n * N, rs_e))
-                fused = None
-            elif defer:
-                state = rt.alloc(16, align=16)
-                state.tensor(torch.int64, (2,)).zero_()
-                push_kw = {"_buf": (recv.offset, state.offset)}
-                if os.environ.get("EDB_RS_LANE", "0") == "1":
-                    push_kw["_lane"] = 1  # wgrad GEMM + pushes on the communication stream
-                tok = graph.call_function(ops.mm_rs_push, args=(a, b, list(ranks)), kwargs=push_kw)
-                pushed.append((tok, recv, state, M // n * N, rs_e))
-                fused = None
-            else:
-                fused = graph.call_function(ops.mm_rs, args=(a, b, list(ranks)),
-                                            kwargs={"_buf": (recv.offset,), "_scale": 1.0 / n})
-        if fused is not None:
-            rs_e.replace_all_uses_with(fused)
-            for dead in [rs_e, rs_s, f] + t_chain + [mm_node]:
-                graph.erase_node(dead)
-        else:
-            # rs_e stays until rs_finish replaces it below; its producers go now
-            rs_e.args = (pushed[-1][0],) + tuple(rs_e.args[1:])
-            for dead in [rs_s, f] + t_chain + [mm_node]:
-                graph.erase_node(dead)
+            tok = graph.call_function(ops.mm_push, args=(a, b, list(ranks)),
+                                      kwargs={"_buf": (recv.offset,)})
+        pushed.append((tok, recv, M // n * N, rs_e))
+        # rs_e stays until rs_finish replaces it below; its producers go now
+        rs_e.args = (tok,) + tuple(rs_e.args[1:])
+        for dead in [rs_s, f] + t_chain + [mm_node]:
+            graph.erase_node(dead)
         n_rs += 1
     if pushed:
         order = {nd: i for i, nd in enumerate(graph.nodes)}
@@ -1669,32 +1646,20 @@ def fuse_collective_gemms(gm, io, rt, ranks, ops=_default_ops, my_index=None):
         groups.append(cur)
         for items in groups:
             with graph.inserting_before(first_use_of(items)):
-                fin_kw = {"_bufs": [(it[1].offset, it[2].offset) if it[2] is not None
-                                    else (it[1].offset,) for it in items],
-                          "_numels": [it[3] for it in items], "_scale": 1.0 / n}
+                fin_kw = {"_bufs": [(it[1].offset,) for it in items],
+                          "_numels": [it[2] for it in items], "_scale": 1.0 / n}
                 toks = [it[0] for it in items]
-                if epoch:
-                    # every member's tiles must have landed before anybody reduces its slots
-                    fin_kw["_epoch"] = 1
-                    toks[0] = graph.call_function(ops.epoch_barrier, args=(toks[0], list(ranks)))
+                # every member's tiles must have landed before anybody reduces its slots
+                toks[0] = graph.call_function(ops.epoch_barrier, args=(toks[0], list(ranks)))
                 fin = graph.call_function(ops.rs_finish, args=(toks, list(ranks)), kwargs=fin_kw)
-                for i, (tok, recv, state, numel, rs_e) in enumerate(items):
+                for i, (tok, recv, numel, rs_e) in enumerate(items):
                     gi = graph.call_function(operator.getitem, args=(fin, i))
                     gi.meta = dict(rs_e.meta)
                     rs_e.replace_all_uses_with(gi)
                     graph.erase_node(rs_e)
 
     # peers read parameter shards in place: keep the optimizer from overwriting them too early
-    if epoch and (rehomed or pushed):
-        insert_epoch_barriers(gm, ranks, ops)
-    elif rehomed:
-        region = optimizer_region(gm, io)
-        if region:
-            anchor = region[0]
-            some_input = next((a_ for a_ in pytree.tree_flatten((anchor.args, anchor.kwargs))[0]
-                               if isinstance(a_, Node)), None)
-            with graph.inserting_before(anchor):
-                graph.call_function(ops.symm_guard, args=(some_input, list(ranks)))
+    insert_epoch_barriers(gm, ranks, ops)
     graph.lint()
     gm.recompile()
     return rehomed, {"ag_mm": n_ag, "ag_pf": n_pf, "mm_rs": n_rs}
@@ -1712,7 +1677,7 @@ def verify_epoch_protocol(gm, ops, n):
       2. every byte of every gathered parameter is prefetched exactly once, by nodes that precede its
          first use; no prefetch item points outside a gathered buffer;
       3. a group barrier separates the last node that reads peers' parameter shards from the first
-         in-place update of such a parameter; every `rs_finish(_epoch=1)` has a barrier between its
+         in-place update of such a parameter; every `rs_finish` has a barrier between its
          last push and itself;
       4. the step ends with a barrier.
 
@@ -1760,7 +1725,7 @@ def verify_epoch_protocol(gm, ops, n):
             if a is not None and b is not None:
                 lo = nd.kwargs["_buf"][0]
                 ranges.append((lo, lo + a.shape[0] * b.shape[1] * 2, f"recv({nd.name})"))
-        elif has("rs_finish") and t is ops.rs_finish and nd.kwargs.get("_epoch"):
+        elif has("rs_finish") and t is ops.rs_finish:
             finishes.append(nd)
         elif has("epoch_barrier") and t is ops.epoch_barrier:
             barriers.append(order[nd])

@@ -423,21 +423,9 @@ def box_exchange(tensor, dst_shape, boxes, peer_src_shapes, group, *, _buf=None)
 
 
 @has_side_effect
-def symm_guard(x, group):
-    """Pass-through that makes the stream wait until no peer is still reading this rank's
-    symmetric buffers (inserted in front of producers that write symmetric memory in place, e.g.
-    the optimizer update of symmetric parameter shards)."""
-    if _is_fake(x) or len(group) <= 1:
-        return x
-    rt, gid, n, _ = _group(group)
-    check(rt.lib.edb_symm_guard(gid, rt.stream()))
-    return x
-
-
-@has_side_effect
 def epoch_barrier(x, group):
     """Pass-through that runs the group-wide epoch barrier on the stream (edb_epoch_barrier).
-    The epoch-mode fused kernels (`ag_mm(_epoch=1)`, `mm_push`) read peers' parameter shards and
+    The fused kernels (`ag_mm`, `mm_push`) read peers' parameter shards and
     write peers' receive slots without any per-op handshake; two of these per train step — one in
     front of the optimizer, one behind it — are the only cross-rank rendezvous left
     (reference: one NCCL rendezvous per collective, sharding.py:94-152)."""
@@ -476,11 +464,16 @@ def gathered(w_shard, group, *deps, _buf):
     return SymmBuffer(rt, int(_buf[1]), n * nbytes).tensor(w_shard.dtype, (n * w_shard.numel(),))
 
 
-def ag_mm(x, w_shard, group, n_out, k_in, bias=None, *, _buf, _epoch=0):
+def ag_mm(x, w_shard, group, n_out, k_in, bias=None, *, _buf, _epoch=1):
     """all_gather(weight shard, dim 0) fused into the consuming GEMM (all_gather_end -> aten.mm /
     addmm of the sharded graph).  `w_shard`: this rank's rows [n_out/n, k_in] (flat or 2-D) living
     at symmetric offset _buf[0]; _buf[1] = offset of the gathered [n_out, k_in] buffer that the
-    kernel's copy CTAs fill while the MMA CTAs already run.  Returns (x @ W^T (+ bias), W_full)."""
+    kernel's copy CTAs fill while the MMA CTAs already run.  Returns (x @ W^T (+ bias), W_full).
+    Epoch protocol: an epoch barrier earlier on the stream made every member's shard final, and
+    none is modified before the next one.  That is the only protocol, so `_epoch` accepts only 1;
+    the keyword is kept for existing callers that pass it."""
+    if _epoch != 1:
+        raise ValueError("ag_mm: only the epoch protocol (_epoch=1) is supported")
     n = len(group)
     if _is_fake(x):
         return (x.new_empty((x.shape[0], n_out)), w_shard.new_empty((n_out, k_in)))
@@ -492,72 +485,21 @@ def ag_mm(x, w_shard, group, n_out, k_in, bias=None, *, _buf, _epoch=0):
     M, K = xc.shape
     assert K == k_in
     out = torch.empty((M, n_out), dtype=torch.bfloat16, device=x.device)
-    if _epoch:
-        from . import gemm as _gemm
-        _gemm.note_fused_call("ag", M, n_out, K, True, True, xc.stride(), (1, k_in), group, _buf)
-    fn = rt.lib.edb_ag_gemm_epoch_bf16 if _epoch else rt.lib.edb_ag_gemm_bf16
-    check(fn(gid, out.data_ptr(), xc.data_ptr(), bias.data_ptr() if bias is not None else None,
-             shard_off, full_off, M, n_out, K, xc.stride(0), n_out, rt.stream()))
+    from . import gemm as _gemm
+    _gemm.note_fused_call("ag", M, n_out, K, True, True, xc.stride(), (1, k_in), group, _buf)
+    check(rt.lib.edb_ag_gemm_epoch_bf16(gid, out.data_ptr(), xc.data_ptr(),
+                                        bias.data_ptr() if bias is not None else None, shard_off,
+                                        full_off, M, n_out, K, xc.stride(0), n_out, rt.stream()))
     w_full = SymmBuffer(rt, full_off, n_out * k_in * 2).tensor(torch.bfloat16, (n_out, k_in))
     return out, w_full
 
 
-def mm_rs(a, b, group, *, _buf, _scale=1.0, _out_dtype=None):
-    """aten.mm fused with reduce_scatter(dim 0): rank r gets rows [r*M/n, (r+1)*M/n) of
-    sum_over_ranks(a @ b) * _scale, flattened (mm -> flatten -> reduce_scatter_start of the
-    zero2/zero3 graphs).  Tiles are TMA-stored straight into the owner's receive slot over NVLink;
-    _buf[0] = symmetric offset of the receive buffer (M*N*2 bytes)."""
-    n = len(group)
-    M, K = a.shape
-    N = b.shape[1]
-    out_dtype = _out_dtype or torch.bfloat16
-    if _is_fake(a):
-        return a.new_empty((M // n * N,), dtype=out_dtype)
-    _require_cuda(a, "mm_rs")
-    from . import gemm as _gemm
-    rt, gid, n, me = _group(group)
-    pa, pb = _gemm._prepare(a, 1), _gemm._prepare(b, 0)
-    if pa is None or pb is None:
-        raise _lib.EdbUnsupported(_lib.EDB_E_UNSUPPORTED, "mm_rs: operand layout")
-    (ta, a_k, lda), (tb, b_k, ldb) = pa, pb
-    out = torch.empty((M // n * N,), dtype=out_dtype, device=a.device)
-    check(rt.lib.edb_gemm_rs_bf16(gid, out.data_ptr(), int(_buf[0]), ta.data_ptr(), tb.data_ptr(),
-                                  M, N, K, lda, ldb, 1 if a_k else 0, 1 if b_k else 0,
-                                  float(_scale), _TORCH_DTYPE_CODE[out_dtype], rt.stream()))
-    return out
-
-
-def mm_rs_push(a, b, group, *, _buf, _lane=0):
-    """Deferred half of mm_rs: computes a @ b and pushes every tile into its owner's receive slot
-    (no waiting, no reduction).  _buf = (symmetric offset of the n receive slots, symmetric offset
-    of 16 zeroed state bytes), both private to this GEMM.  Returns an empty token that `rs_finish`
-    takes so that the graph keeps the order.  `_lane=1`: the kernel runs on the communication
-    stream (own group / op sequence), so the weight-gradient GEMM and its pushes overlap the
-    data-gradient GEMM that follows on the compute stream; rs_finish joins."""
-    if _is_fake(a):
-        return a.new_empty((0,))
-    _require_cuda(a, "mm_rs_push")
-    from . import gemm as _gemm
-    rt, gid, n, me = _group(group, _lane)
-    M, K = a.shape
-    N = b.shape[1]
-    pa, pb = _gemm._prepare(a, 1), _gemm._prepare(b, 0)
-    if pa is None or pb is None:
-        raise _lib.EdbUnsupported(_lib.EDB_E_UNSUPPORTED, "mm_rs_push: operand layout")
-    (ta, a_k, lda), (tb, b_k, ldb) = pa, pb
-    token = torch.empty((0,), dtype=a.dtype, device=a.device)
-    with _Lane(_lane and n > 1) as lane:
-        check(rt.lib.edb_gemm_rs_push_bf16(gid, int(_buf[0]), int(_buf[1]), ta.data_ptr(),
-                                           tb.data_ptr(), M, N, K, lda, ldb, 1 if a_k else 0,
-                                           1 if b_k else 0, rt.stream()))
-    return lane.tag(token, ta, tb)
-
-
 def mm_push(a, b, group, *, _buf):
-    """Epoch-mode push half of mm_rs: a @ b on the regular GEMM path (cta_group::2 pairs, split-K)
-    with every row block stored into its owner's receive slot over NVLink; no flags at all — the
-    epoch barrier in front of `rs_finish(_epoch=1)` makes the slots complete.  _buf = (symmetric
-    offset of the n receive slots,).  Returns an empty token for graph ordering."""
+    """aten.mm whose result is reduce-scattered over its rows (mm -> flatten ->
+    reduce_scatter_start of the zero2/zero3 graphs), push half: a @ b on the regular GEMM path
+    (cta_group::2 pairs, split-K) with every row block stored into its owner's receive slot over
+    NVLink; no flags at all — the epoch barrier in front of `rs_finish` makes the slots complete.
+    _buf = (symmetric offset of the n receive slots,).  Returns an empty token for graph ordering."""
     if _is_fake(a):
         return a.new_empty((0,))
     _require_cuda(a, "mm_push")
@@ -575,37 +517,27 @@ def mm_push(a, b, group, *, _buf):
     return torch.empty((0,), dtype=a.dtype, device=a.device)
 
 
-def rs_finish(tokens, group, *, _bufs, _numels, _scale=1.0, _out_dtype=None, _epoch=0):
+def rs_finish(tokens, group, *, _bufs, _numels, _scale=1.0, _out_dtype=None):
     """Reduce the receive slots of the pushed GEMMs `tokens` came from, all in one kernel:
     item i -> flat shard of _numels[i] elements = sum over ranks (rank order, fp32) * _scale.
-    _bufs[i] = the (_buf) pair given to mm_rs_push i."""
+    _bufs[i] = the (_buf) given to mm_push i.  The caller puts an epoch barrier in front: every
+    slot is complete, nothing to wait for."""
     out_dtype = _out_dtype or torch.bfloat16
     if tokens and _is_fake(tokens[0]):
         return [tokens[0].new_empty((int(k),), dtype=out_dtype) for k in _numels]
-    lane_id = 1 if any(hasattr(t, "_edb_pending") for t in tokens) else 0
-    for t in tokens:
-        _join(t)  # pushes issued on the communication lane: wait for them on this stream
-    # the reduction belongs to the op sequence the pushes ran in
-    rt, gid, n, me = _group(group, lane_id)
+    rt, gid, n, me = _group(group)
     dev = tokens[0].device
     outs = [torch.empty((int(k),), dtype=out_dtype, device=dev) for k in _numels]
     cnt = len(outs)
     dsts = (ctypes.c_void_p * cnt)(*[o.data_ptr() for o in outs])
     recv = (ctypes.c_uint64 * cnt)(*[int(b[0]) for b in _bufs])
-    state = (ctypes.c_uint64 * cnt)(*[int(b[1]) if len(b) > 1 else 0 for b in _bufs])
     chunk = (ctypes.c_int64 * cnt)(*[int(k) * 2 for k in _numels])  # slots hold bf16
-    if _epoch:
-        # the caller put an epoch barrier in front: every slot is complete, nothing to wait for
-        check(rt.lib.edb_rs_finish_local(gid, cnt, dsts, recv, chunk, float(_scale),
-                                         _TORCH_DTYPE_CODE[out_dtype], rt.stream()))
-    else:
-        check(rt.lib.edb_rs_finish(gid, cnt, dsts, recv, state, chunk, float(_scale),
-                                   _TORCH_DTYPE_CODE[out_dtype], rt.stream()))
+    check(rt.lib.edb_rs_finish_local(gid, cnt, dsts, recv, chunk, float(_scale),
+                                     _TORCH_DTYPE_CODE[out_dtype], rt.stream()))
     return outs
 
 
 COMM_FUNCS = [all_reduce_start, all_gather_start, reduce_scatter_start, all_to_all_start]
 COMM_SYNC_FUNCS = [all_reduce_end, all_gather_end, reduce_scatter_end, all_to_all_end]
 CUSTOM_FUNCS = COMM_FUNCS + COMM_SYNC_FUNCS + [scatter_wrapper, copy_wrapper]
-FUSED_FUNCS = [ag_mm, mm_rs, mm_rs_push, mm_push, rs_finish, symm_guard, epoch_barrier, ag_prefetch,
-               gathered]
+FUSED_FUNCS = [ag_mm, mm_push, rs_finish, epoch_barrier, ag_prefetch, gathered]

@@ -152,12 +152,6 @@ int edb_halo_exchange(int gid, void* dst, uint64_t stage_off, const void* src,
                       const int64_t* local_shape, int ndim, int dim, int halo, int elem_size,
                       void* stream);
 
-/* Producer-side guard: make the stream wait until every peer has finished reading this rank's
- * symmetric buffers from earlier collectives (write-after-read), then — when `signal` != 0 —
- * publish "my symmetric data for the next op is ready" without moving data.  Used by fused
- * producers (GEMM epilogues, optimizer updates) that write symmetric memory themselves. */
-int edb_symm_guard(int gid, void* stream);
-
 /* ---- dense compute on the path (sharded-op kernel dispatch) ------------------------------- */
 
 /* C[M,N] (bf16, row-major, ldc) = A·B (+ bias) with fp32 accumulation on tcgen05 tensor cores.
@@ -186,40 +180,6 @@ int edb_gemm_epi_bf16(void* C, const void* A, const void* B, const void* bias, c
                       const uint64_t* src_offs, const uint64_t* dst_offs, const int64_t* bytes,
                       const int64_t* dst_strides, const int64_t* src_strides, void* stream);
 
-/* all-gather fused into the consuming GEMM: B (weights [N,K], K-major) is sharded S(0) over the
- * group, shard (N/n rows) resident at symmetric offset `b_shard_off` on every rank.  The kernel's
- * copy CTAs pull the peer shards into the local gathered buffer `b_full_off` chunk by chunk while
- * the MMA CTAs start on the local shard and consume chunks as their flags arrive.
- * C[M,N] = A[M,K]·B_fullᵀ.  (all_gather_end -> aten.mm pattern, SURVEY App. B) */
-int edb_ag_gemm_bf16(int gid, void* C, const void* A, const void* bias, uint64_t b_shard_off,
-                     uint64_t b_full_off, int64_t M, int64_t N, int64_t K, int64_t lda, int64_t ldc,
-                     void* stream);
-
-/* GEMM fused with reduce-scatter: partial C[M,N] = A·B is produced tile by tile into the
- * symmetric stage `c_stage_off` (row-chunks destined for other ranks first); reduce CTAs of the
- * owner pull each finished chunk from every peer, sum in rank order, scale and cast into `dst`
- * ([M/n, N], out_dtype).  (aten.mm -> reduce_scatter_start pattern.) */
-int edb_gemm_rs_bf16(int gid, void* dst, uint64_t c_stage_off, const void* A, const void* B,
-                     int64_t M, int64_t N, int64_t K, int64_t lda, int64_t ldb, int a_kmajor,
-                     int b_kmajor, float post_scale, int out_dtype, void* stream);
-
-/* Deferred form of the fused GEMM + reduce-scatter (weight gradients of zero2/zero3: the reduced
- * shard is only needed by the optimizer at the end of the step).  `edb_gemm_rs_push_bf16` computes
- * C = A.B and TMA-stores every tile into the owner's receive slot [me] (symmetric `recv_off`, n
- * slots of (M/n)*N*2 bytes, dedicated to this GEMM) without waiting for anybody: no lockstep with
- * the peers and no tail.  `state_off`: 16 zero-initialised symmetric bytes private to this GEMM
- * (word 0: op number of the push, word 1: op number of the last reduction — the push checks the
- * owners' DONE flags against it, which guards the slots across steps).  `edb_rs_finish` reduces the
- * slots of n_items such GEMMs in ONE launch (rank order, fp32, scale, cast; host arrays of
- * per-item destinations, offsets and slot sizes), waiting once for every source's latest push.
- * Result identical to edb_gemm_rs_bf16. */
-int edb_gemm_rs_push_bf16(int gid, uint64_t recv_off, uint64_t state_off, const void* A,
-                          const void* B, int64_t M, int64_t N, int64_t K, int64_t lda, int64_t ldb,
-                          int a_kmajor, int b_kmajor, void* stream);
-int edb_rs_finish(int gid, int n_items, void* const* dsts, const uint64_t* recv_offs,
-                  const uint64_t* state_offs, const int64_t* chunk_bytes, float post_scale,
-                  int out_dtype, void* stream);
-
 /* ---- epoch protocol: one group barrier per phase of the step instead of a handshake per op ----
  *
  * The per-op protocol above costs several dependent system-scope round trips per collective
@@ -237,9 +197,13 @@ int edb_rs_finish(int gid, int n_items, void* const* dsts, const uint64_t* recv_
  * visible to every member after it (system-scope fence + release / acquire). */
 int edb_epoch_barrier(int gid, void* stream);
 
-/* edb_ag_gemm_bf16 without the per-op handshake: the caller guarantees, with an
- * edb_epoch_barrier earlier on every member's stream, that all shards at `b_shard_off` are final,
- * and that nobody modifies its shard before the next barrier.  Same result. */
+/* All-gather fused into the consuming GEMM: B (weights [N,K], K-major) is sharded S(0) over the
+ * group, shard (N/n rows) resident at symmetric offset `b_shard_off` on every rank.  The kernel's
+ * copy CTAs pull the peer shards into the local gathered buffer `b_full_off` while the MMA CTAs
+ * start on the local shard and consume the others as the copy CTAs announce them (local flags
+ * only).  C[M,N] = A[M,K]·B_fullᵀ.  (all_gather_end -> aten.mm pattern, SURVEY App. B)
+ * The caller guarantees, with an edb_epoch_barrier earlier on every member's stream, that all
+ * shards at `b_shard_off` are final, and that nobody modifies its shard before the next barrier. */
 int edb_ag_gemm_epoch_bf16(int gid, void* C, const void* A, const void* bias, uint64_t b_shard_off,
                            uint64_t b_full_off, int64_t M, int64_t N, int64_t K, int64_t lda,
                            int64_t ldc, void* stream);

@@ -115,12 +115,8 @@ def all_to_all_end(tensor, gather_dim, scatter_dim, num_chunks, indice, ranks, t
     return tensor
 
 
-# fused ops (semantics of easydist_b200.reshard.ag_mm / mm_rs / symm_guard) for CPU tests of the
+# fused ops (semantics of easydist_b200.reshard.ag_mm / mm_push / rs_finish) for CPU tests of the
 # fusion rewrite
-
-
-def symm_guard(x, group):
-    return x
 
 
 _EPOCHS = {"barriers": 0, "open_pushes": 0}
@@ -156,7 +152,7 @@ def mm_push(a, b, group, *, _buf=None):
     return a @ b
 
 
-def ag_mm(x, w_shard, group, n_out, k_in, bias=None, *, _buf=None, _epoch=0):
+def ag_mm(x, w_shard, group, n_out, k_in, bias=None, *, _buf=None, _epoch=1):
     if _fake(x):
         return x.new_empty((x.shape[0], n_out)), w_shard.new_empty((n_out, k_in))
     w = all_gather_start(w_shard.reshape(-1), 0, group).view(n_out, k_in)
@@ -166,31 +162,12 @@ def ag_mm(x, w_shard, group, n_out, k_in, bias=None, *, _buf=None, _epoch=0):
     return out, w
 
 
-def mm_rs(a, b, group, *, _buf=None, _scale=1.0, _out_dtype=None):
-    n = len(group)
-    if _fake(a):
-        return a.new_empty((a.shape[0] // n * b.shape[1],), dtype=_out_dtype or a.dtype)
-    part = (a @ b).flatten()
-    red = all_reduce_start(part, "sum", group)
-    me = list(group).index(dist.get_rank())
-    out = torch.chunk(red, n, 0)[me].contiguous() * _scale
-    return out.to(_out_dtype or a.dtype)
-
-
-def mm_rs_push(a, b, group, *, _buf=None, _lane=0):
-    """CPU stand-in of reshard.mm_rs_push: the 'token' carries the partial product itself."""
-    if _fake(a):
-        return a.new_empty((a.shape[0], b.shape[1]))
-    return a @ b
-
-
-def rs_finish(tokens, group, *, _bufs=None, _numels=None, _scale=1.0, _out_dtype=None, _epoch=0):
+def rs_finish(tokens, group, *, _bufs=None, _numels=None, _scale=1.0, _out_dtype=None):
     n = len(group)
     if tokens and _fake(tokens[0]):
         return [t.new_empty((int(k),), dtype=_out_dtype or t.dtype) for t, k in zip(tokens, _numels)]
-    if _epoch:
-        # epoch protocol: a barrier must separate the pushes from their reduction
-        assert _EPOCHS["open_pushes"] == 0, "rs_finish(_epoch=1) without an epoch barrier in front"
+    # epoch protocol: a barrier must separate the pushes from their reduction
+    assert _EPOCHS["open_pushes"] == 0, "rs_finish without an epoch barrier in front"
     me = list(group).index(dist.get_rank())
     outs = []
     for t in tokens:
@@ -246,8 +223,7 @@ class FakeSymmRuntime:
         return FakeSymmRuntime._Buf(off, nbytes)
 
 
-FUSED_FUNCS = [ag_mm, mm_rs, mm_rs_push, mm_push, rs_finish, symm_guard, epoch_barrier, ag_prefetch,
-               gathered]
+FUSED_FUNCS = [ag_mm, mm_push, rs_finish, epoch_barrier, ag_prefetch, gathered]
 COMM_FUNCS = [all_reduce_start, all_gather_start, reduce_scatter_start, all_to_all_start]
 COMM_SYNC_FUNCS = [all_reduce_end, all_gather_end, reduce_scatter_end, all_to_all_end]
 CUSTOM_FUNCS = COMM_FUNCS + COMM_SYNC_FUNCS + [scatter_wrapper, copy_wrapper]

@@ -358,122 +358,6 @@ def run_graph(rank, world, group, rows=64):
     return 5
 
 
-def run_fused(rank, world, group):
-    """Fused all-gather+GEMM and GEMM+reduce-scatter vs the unfused kernels: bit-exact (same
-    tile math, same reduction order)."""
-    from easydist_b200 import gemm
-    rt = runtime.get_runtime()
-    n_ok = 0
-    # the unfused references below must accumulate in the same order as the fused kernels, which
-    # never split K
-    rt.set_option("gemm_splitk", 0)
-    try:
-        n_ok += _run_fused_cases(rank, world, group, rt, gemm)
-    finally:
-        rt.set_option("gemm_splitk", 1)
-    n_ok += run_deferred_rs(rank, world, group)
-    return n_ok
-
-
-def _run_fused_cases(rank, world, group, rt, gemm):
-    n_ok = 0
-    torch.manual_seed(1234)  # same on every rank: every rank knows every shard
-    for (M, N, K, with_bias) in [(512, 256 * world, 256, False), (4096, 1024, 1024, True),
-                                 (384, 128 * world, 1000 // 8 * 8, False), (4096, 4096, 1024, True)]:
-        if N % world or N % 128:
-            continue
-        W = (torch.randn(N, K, device="cuda") * 0.1).bfloat16()
-        x = torch.randn(M, K, device="cuda").bfloat16()
-        bias = torch.randn(N, device="cuda").bfloat16() if with_bias else None
-        rows = N // world
-        shard_buf = rt.alloc(rows * K * 2, align=1024)
-        full_buf = rt.alloc(N * K * 2, align=1024)
-        w_shard = shard_buf.tensor(torch.bfloat16, (rows, K))
-        for it in range(3):  # repeated: WAR guard + epochs
-            w_shard.copy_(W[rank * rows:(rank + 1) * rows] * (it + 1))
-            reshard.symm_guard(w_shard, group)
-            out, w_full = reshard.ag_mm(x, w_shard, group, N, K, bias,
-                                        _buf=(shard_buf.offset, full_buf.offset))
-            Wi = W * (it + 1)
-            ref = gemm.addmm(bias, x, Wi.t()) if with_bias else gemm.mm(x, Wi.t())
-            assert torch.equal(w_full, Wi), f"ag_mm gathered weight mismatch {(M, N, K)} it {it}"
-            assert torch.equal(out, ref), f"ag_mm output mismatch {(M, N, K)} it {it}: " \
-                f"{(out.float() - ref.float()).abs().max()}"
-            n_ok += 1
-    for (M, N, K) in [(128 * world, 256, 512), (1024, 1024, 4096), (4096, 1024, 4096),
-                      (256 * world, 4096, 1024)]:
-        if (M // world) % 128:
-            continue
-        g = torch.Generator(device="cuda").manual_seed(77)
-        a_all = [torch.randn(K, M, device="cuda", generator=g).bfloat16() for _ in range(world)]
-        b_all = [torch.randn(K, N, device="cuda", generator=g).bfloat16() for _ in range(world)]
-        recv = rt.alloc(M * N * 2, align=1024)
-        stage = rt.alloc(M * N * 2, align=1024)
-        for it in range(3):
-            a = a_all[rank].t()        # [M,K] column-major (dy^T of a wgrad)
-            b = b_all[rank]            # [K,N] row-major
-            got = reshard.mm_rs(a, b, group, _buf=(recv.offset,), _scale=1.0 / world)
-            part = gemm.mm(a, b)
-            want = reshard.reduce_scatter_start(part.flatten(), "avg", 0, group,
-                                                _buf=(stage.offset, M * N * 2))
-            assert torch.equal(got, want), f"mm_rs mismatch {(M, N, K)} it {it}: " \
-                f"{(got.float() - want.float()).abs().max()}"
-            n_ok += 1
-    return n_ok
-
-
-def run_deferred_rs(rank, world, group):
-    """Deferred GEMM+RS (mm_rs_push x k, other ops in between, then ONE rs_finish) vs mm_rs: bit
-    exact, over several steps (the cross-step slot guard) and from a replayed CUDA graph."""
-    from easydist_b200 import gemm
-    rt = runtime.get_runtime()
-    shapes = [(M, N, K) for (M, N, K) in [(128 * world, 256, 512), (1024, 1024, 4096),
-                                          (1024, 4096, 4096), (256 * world, 3072, 1024)]
-              if (M // world) % 128 == 0]
-    g = torch.Generator(device="cuda").manual_seed(99)
-    data = []
-    for (M, N, K) in shapes:
-        a_all = [torch.randn(K, M, device="cuda", generator=g).bfloat16() for _ in range(world)]
-        b_all = [torch.randn(K, N, device="cuda", generator=g).bfloat16() for _ in range(world)]
-        recv, recv2 = rt.alloc(M * N * 2, align=1024), rt.alloc(M * N * 2, align=1024)
-        state = rt.alloc(16, align=16)
-        state.tensor(torch.int64, (2,)).zero_()
-        data.append((a_all[rank], b_all[rank].clone(), recv, recv2, state))
-    scale_in = torch.ones((), device="cuda", dtype=torch.bfloat16)
-
-    def step():
-        toks, wants = [], []
-        for (M, N, K), (a_t, b, recv, recv2, state) in zip(shapes, data):
-            bb = b * scale_in  # new values every step, same addresses under graph replay
-            toks.append(reshard.mm_rs_push(a_t.t(), bb, group, _buf=(recv.offset, state.offset)))
-            wants.append(reshard.mm_rs(a_t.t(), bb, group, _buf=(recv2.offset,), _scale=1.0 / world))
-        outs = reshard.rs_finish(toks, group, _bufs=[(d[2].offset, d[4].offset) for d in data],
-                                 _numels=[M // world * N for (M, N, K) in shapes], _scale=1.0 / world)
-        return outs, wants
-
-    n_ok = 0
-    for it in range(3):
-        scale_in.fill_(float(it + 1))
-        outs, wants = step()
-        torch.cuda.synchronize()
-        for o, w, shp in zip(outs, wants, shapes):
-            assert torch.equal(o, w), f"deferred rs mismatch {shp} it {it}: " \
-                f"{(o.float() - w.float()).abs().max()}"
-            n_ok += 1
-    graph = torch.cuda.CUDAGraph()
-    with torch.cuda.graph(graph):
-        outs, wants = step()
-    for it in range(4):
-        scale_in.fill_(float(2 * it + 1))
-        graph.replay()
-        torch.cuda.synchronize()
-        for o, w, shp in zip(outs, wants, shapes):
-            assert torch.equal(o, w), f"deferred rs (graph) mismatch {shp} replay {it}"
-            n_ok += 1
-    assert not any(rt.error_flags()), rt.error_flags()
-    return n_ok
-
-
 def run_epoch(rank, world, group):
     """Epoch protocol (edb_epoch_barrier + flag-free fused kernels): a miniature train step
 
@@ -482,19 +366,21 @@ def run_epoch(rank, world, group):
 
     repeated eagerly and from a replayed CUDA graph, with artificial rank skew (busy-wait kernels
     on alternating ranks) so that a missing rendezvous shows up as stale data.  Checked (i) bit for
-    bit against the unfused kernels of this library (plain GEMM; GEMM -> reduce_scatter(avg) with
-    the per-op flag protocol) and (ii) against a plain fp32 PyTorch computation of the same
-    products (relative L2 error <= 6e-3: one bf16 rounding of the product / of each rank's partial
-    product, 2^-9 rms)."""
+    bit against the unfused kernels of this library (plain GEMM without split-K, like the fused
+    kernel; GEMM -> reduce_scatter(avg) with the per-op flag protocol) and (ii) against a plain
+    fp32 PyTorch computation of the same products (relative L2 error <= 6e-3: one bf16 rounding of
+    the product / of each rank's partial product, 2^-9 rms).  The shapes include a K tail
+    (K = 1000) and a reduce-scatter whose rows per rank are not a multiple of the tile pair."""
     from easydist_b200 import gemm
     rt = runtime.get_runtime()
     torch.manual_seed(4321)  # same on every rank: every rank knows every rank's operands
     ag_cases = [(M, N, K, wb) for (M, N, K, wb) in
                 [(512, 256 * world, 256, False), (4096, 1024, 1024, True), (4096, 4096, 1024, True),
-                 (4096, 3072, 1024, True)] if N % world == 0 and N % 128 == 0 and (N // world) % 8 == 0]
+                 (4096, 3072, 1024, True), (384, 128 * world, 1000, False)]
+                if N % world == 0 and N % 128 == 0 and (N // world) % 8 == 0]
     rs_cases = [(M, N, K) for (M, N, K) in
                 [(128 * world, 256, 512), (1024, 1024, 4096), (4096, 1024, 4096), (1024, 4096, 4096),
-                 (3072, 1024, 4096)] if (M // world) % 128 == 0]
+                 (3072, 1024, 4096), (256 * world, 4096, 1024)] if (M // world) % 128 == 0]
     ag = []
     for (M, N, K, with_bias) in ag_cases:
         W = (torch.randn(N, K, device="cuda") * 0.1).bfloat16()
@@ -527,7 +413,7 @@ def run_epoch(rank, world, group):
         for (N_, (W, x, bias, shard_buf, full_buf, w_shard)) in zip(ag_cases, ag):
             M, N, K, _ = N_
             o, wf = reshard.ag_mm(x, w_shard, group, N, K, bias,
-                                  _buf=(shard_buf.offset, full_buf.offset), _epoch=1)
+                                  _buf=(shard_buf.offset, full_buf.offset))
             outs.append(o)
             fulls.append(wf.clone())
         maybe_sleep(1)
@@ -541,7 +427,7 @@ def run_epoch(rank, world, group):
         toks[0] = reshard.epoch_barrier(toks[0], group)
         reds = reshard.rs_finish(toks, group, _bufs=[(r_[2].offset,) for r_ in rs],
                                  _numels=[M // world * N for (M, N, K) in rs_cases],
-                                 _scale=1.0 / world, _epoch=1)
+                                 _scale=1.0 / world)
         maybe_sleep(1)
         # the "optimizer": every rank rewrites its symmetric weight shard in place
         factor.add_(1)
@@ -556,7 +442,12 @@ def run_epoch(rank, world, group):
         for (M, N, K, with_bias), (W, x, bias, *_), o, wf in zip(ag_cases, ag, outs, fulls):
             Wi = (W * torch.tensor(it_factor, dtype=torch.bfloat16, device="cuda"))
             assert torch.equal(wf, Wi), f"{what}: epoch ag_mm gathered weight {(M, N, K)} x{it_factor}"
-            ref = gemm.addmm(bias, x, Wi.t()) if with_bias else gemm.mm(x, Wi.t())
+            # the fused kernel never splits K: neither may its reference
+            rt.set_option("gemm_splitk", 0)
+            try:
+                ref = gemm.addmm(bias, x, Wi.t()) if with_bias else gemm.mm(x, Wi.t())
+            finally:
+                rt.set_option("gemm_splitk", 1)
             assert torch.equal(o, ref), f"{what}: epoch ag_mm {(M, N, K)} x{it_factor}: " \
                 f"{(o.float() - ref.float()).abs().max()}"
             f32 = x.float() @ Wi.float().t() + (bias.float() if with_bias else 0.0)
@@ -757,7 +648,7 @@ def bench_fused(rank, world, group):
         w_shard = shard_buf.tensor(torch.bfloat16, (rows, K))
         w_shard.normal_()
         t_fused = timeit(lambda: reshard.ag_mm(x, w_shard, group, N, K, None,
-                                                _buf=(shard_buf.offset, full_buf.offset)))
+                                                _buf=(shard_buf.offset, full_buf.offset), _epoch=1))
 
         def unfused():
             w = reshard.all_gather_start(w_shard, 0, group, _buf=(ag_buf.offset, N * K * 2))
@@ -766,16 +657,7 @@ def bench_fused(rank, world, group):
         t_gemm = timeit(lambda: gemm.mm(x, full_buf.tensor(torch.bfloat16, (N, K)).t()))
         # wgrad-like: dW[N,K] = dy^T[N,M] @ x[M,K], reduce-scattered over N
         dy = torch.randn(M, N, device="cuda").bfloat16()
-        recv, stage = rt.alloc(N * K * 2, align=1024), rt.alloc(N * K * 2, align=1024)
-        t_rs_f = timeit(lambda: reshard.mm_rs(dy.t(), x, group, _buf=(recv.offset,), _scale=1.0 / world))
-        st8 = rt.alloc(16, align=16)
-        st8.tensor(torch.int64, (2,)).zero_()
-
-        def deferred():
-            tok = reshard.mm_rs_push(dy.t(), x, group, _buf=(recv.offset, st8.offset))
-            return reshard.rs_finish([tok], group, _bufs=[(recv.offset, st8.offset)],
-                                     _numels=[N // world * K], _scale=1.0 / world)
-        t_rs_d = timeit(deferred)
+        stage = rt.alloc(N * K * 2, align=1024)
         t_wg = timeit(lambda: gemm.mm(dy.t(), x))
 
         def unfused_rs():
@@ -785,8 +667,8 @@ def bench_fused(rank, world, group):
         t_rs_u = timeit(unfused_rs)
         if rank == 0:
             print(f"FUSED M{M} N{N} K{K}: ag+gemm fused {t_fused:.1f}us unfused {t_unf:.1f}us "
-                  f"(gemm alone {t_gemm:.1f}us) | gemm+rs fused {t_rs_f:.1f}us unfused {t_rs_u:.1f}us "
-                  f"push+finish {t_rs_d:.1f}us (wgrad gemm alone {t_wg:.1f}us)", flush=True)
+                  f"(gemm alone {t_gemm:.1f}us) | gemm+rs unfused {t_rs_u:.1f}us "
+                  f"(wgrad gemm alone {t_wg:.1f}us)", flush=True)
 
 
 def run_lane(rank, world, group):
@@ -1098,7 +980,6 @@ def main():
     n += run_p2p(rank, world, group)
     n += run_graph(rank, world, group)
     n += run_graph(rank, world, group, rows=4)
-    n += run_fused(rank, world, group)
     n += run_epoch(rank, world, group)
     n += run_prefetch(rank, world, group)
     n += run_push_cases(rank, world, group)

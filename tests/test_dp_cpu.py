@@ -71,12 +71,9 @@ class Wide(torch.nn.Module):
         return self.fc2(torch.nn.functional.gelu(self.fc1(self.norm(x))))
 
 
-def _fusion_worker(rank, world, port, q, defer="0", d=256):
+def _fusion_worker(rank, world, port, q, case="epoch", d=256):
     os.environ["OMP_NUM_THREADS"] = "1"
-    os.environ["EDB_EPOCH"] = "1" if defer == "epoch" else "0"
-    defer = "0" if defer == "epoch" else defer
-    os.environ["EDB_DEFER_RS"] = defer
-    os.environ["EDB_RS_LANE"] = defer  # deferred pushes also go to the communication lane
+    os.environ["EDB_AG_PREFETCH"] = "0" if case == "no_prefetch" else "1"
     torch.set_num_threads(1)
     dist.init_process_group("gloo", init_method=f"tcp://127.0.0.1:{port}", rank=rank,
                             world_size=world)
@@ -106,9 +103,6 @@ def _fusion_worker(rank, world, port, q, defer="0", d=256):
         if not torch.allclose(loss_all, ref_loss.detach().float(), rtol=3e-2, atol=1e-3):
             ok, msg = False, f"loss {loss_all} vs {ref_loss}"
     info = dict(compiled.info)
-    info["lane_pushes"] = sum(1 for n in compiled.graph.graph.nodes
-                              if n.op == "call_function" and n.target is gloo_ops.mm_rs_push
-                              and n.kwargs.get("_lane") == 1)
     info["barriers_run"] = gloo_ops._EPOCHS["barriers"]
     nodes = list(compiled.graph.graph.nodes)
     info["order"] = [n.target.__name__ for n in nodes if n.op == "call_function" and
@@ -121,43 +115,40 @@ def _fusion_worker(rank, world, port, q, defer="0", d=256):
     dist.destroy_process_group()
 
 
-@pytest.mark.parametrize("defer,world,d", [("0", 2, 256), ("1", 2, 256), ("epoch", 2, 256),
-                                           ("epoch", 4, 512)])
-def test_fusion_rewrite_on_cpu(defer, world, d):
+@pytest.mark.parametrize("case,world,d", [("epoch", 2, 256), ("epoch", 4, 512),
+                                          ("no_prefetch", 2, 256), ("no_prefetch", 4, 512)])
+def test_fusion_rewrite_on_cpu(case, world, d):
     """The AG+GEMM / GEMM+RS peephole (lowering.fuse_collective_gemms) rewrites the zero3 graph of
-    a 2-layer MLP: both weights' all-gathers fuse into their forward GEMMs and both weight
-    gradients' reduce-scatters fuse into the wgrad GEMMs (defer=1: push-only GEMMs + one rs_finish
-    in front of the optimizer); training still matches vanilla."""
+    a 2-layer MLP: both weight gradients' reduce-scatters become push-only GEMMs + one rs_finish in
+    front of the optimizer, and both weights' all-gathers become prefetches (no_prefetch: fuse into
+    their forward GEMMs, ag_mm); training still matches vanilla."""
     ok, msg, info = run_world(_fusion_worker, world,
-                              lambda r, port, q: (r, world, port, q, defer, d), timeout=180)
+                              lambda r, port, q: (r, world, port, q, case, d), timeout=180)
     assert ok, msg
-    want_fused = {"ag_mm": 0, "ag_pf": 2, "mm_rs": 2} if defer == "epoch" else \
+    want_fused = {"ag_mm": 0, "ag_pf": 2, "mm_rs": 2} if case == "epoch" else \
         {"ag_mm": 2, "ag_pf": 0, "mm_rs": 2}
     assert info["fused"] == want_fused, info
     assert info["comm_nodes"].get("reduce_scatter_start", 0) == 0, info
-    if defer == "epoch":
-        # epoch protocol: flag-free fused kernels, exactly two barriers per step — one between the
-        # last push and the reduction of the slots (in front of the optimizer), one at the very end
-        assert info["comm_nodes"].get("mm_push") == 2 and info["comm_nodes"].get("rs_finish") == 1, info
-        assert info["comm_nodes"].get("epoch_barrier") == 2, info
-        assert "symm_guard" not in info["comm_nodes"] and "mm_rs" not in info["comm_nodes"], info
+    # epoch protocol: flag-free fused kernels, exactly two barriers per step — one between the
+    # last push and the reduction of the slots (in front of the optimizer), one at the very end
+    assert info["comm_nodes"].get("mm_push") == 2 and info["comm_nodes"].get("rs_finish") == 1, info
+    assert info["comm_nodes"].get("epoch_barrier") == 2, info
+    assert info["barriers_run"] == 2 * 3, info  # 3 steps
+    order = info["order"]
+    if case == "epoch":
         # parameter gathers are prefetches: fc1's (needed before the first GEMM) stand-alone at the
         # top, fc2's riding on the fc1 GEMM up to that (tiny) GEMM's byte budget and the remainder
         # stand-alone in front of the use; every use reads the gathered buffer
         assert info["comm_nodes"].get("ag_prefetch") == 2 and "ag_mm" not in info["comm_nodes"], info
         assert info["comm_nodes"].get("gathered", 0) >= 2, info
         assert info["carried"] == 1, info
-        order = info["order"]
         assert order.index("rs_finish") == order.index("epoch_barrier") + 1, order
         assert max(i for i, k in enumerate(order) if k == "mm_push") < order.index("epoch_barrier"), order
         assert order[-1] == "epoch_barrier", order
-        assert info["barriers_run"] == 2 * 3, info  # 3 steps
-    elif defer == "1":
-        assert info["comm_nodes"].get("mm_rs_push") == 2 and info["comm_nodes"].get("rs_finish") == 1, info
-        assert "mm_rs" not in info["comm_nodes"], info
-        assert info["lane_pushes"] == 2, info
     else:
-        assert info["comm_nodes"].get("mm_rs") == 2, info
+        assert info["comm_nodes"].get("ag_mm") == 2, info
+        assert order == ["ag_mm", "ag_mm", "mm_push", "mm_push", "epoch_barrier", "rs_finish",
+                         "epoch_barrier"], order
 
 
 def _run_case(rank, world, mode, opt_kind, bucket=0, generic_bucket="0", overlap="0", clip=False):

@@ -29,7 +29,6 @@ class Deep(torch.nn.Module):
 @pytest.mark.parametrize("gbps,my_index", [("300", 1), ("0.001", 0), ("100000", None)])
 def test_every_shard_byte_is_prefetched_once_before_its_first_use(gbps, my_index, monkeypatch):
     monkeypatch.setenv("EDB_PF_GBPS", gbps)
-    monkeypatch.setenv("EDB_EPOCH", "1")
     from easydist_b200 import lowering
     from easydist_b200.api import _flat_inputs
     from easydist_b200.compile import GraphIO, trace_train_step
@@ -113,7 +112,6 @@ def test_static_buffers_mark_push_collectives_and_the_step_ends_with_a_barrier(m
     """lowering.assign_static_buffers(push=True): every remaining collective node of the zero3 graph
     gets dedicated symmetric buffers and `_push=1`; an all-reduce's receive buffer follows the
     one-shot / two-shot rule of edb_all_reduce_push; ensure_end_barrier is idempotent."""
-    monkeypatch.setenv("EDB_EPOCH", "1")
     from easydist_b200 import lowering
     from easydist_b200.api import _flat_inputs
     from easydist_b200.compile import GraphIO, trace_train_step
@@ -197,7 +195,6 @@ def test_static_epoch_protocol_check_passes_and_catches_planted_races(monkeypatc
     compile_auto.py:269-351): the lowered zero3 graph satisfies the contract; a removed barrier, two
     nodes sharing a receive buffer, a dropped prefetch range and a prefetch after the first use are
     each reported."""
-    monkeypatch.setenv("EDB_EPOCH", "1")
     from easydist_b200 import lowering
     from tests import gloo_ops
     gm, ranks = _lowered_zero3_graph()
