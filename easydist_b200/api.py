@@ -100,27 +100,7 @@ def _finish(gm, params, buffers, named_states, args, kwargs, ops, native, io=Non
         # opt-in: changes the communication structure the reference's lowering would produce
         info["bucketed"] = lowering.bucket_small_comm(gm, ops)
         lowering.propagate_local_meta(gm, flat)
-    experimental = [k for k in ("EDB_OVERLAP", "EDB_GEMM_SIDE")
-                    if os.environ.get(k, "0") == "1"]
-    if experimental and native:
-        # round-1 advisor finding: kernels whose CTAs wait on other CTAs assume the whole grid is
-        # co-resident, which a second stream breaks (resident CTAs would wait on CTAs that cannot be
-        # scheduled until the fatal timeout fires).  Gated until the spinning kernels are launched
-        # cooperatively / sized from the SMs actually free.
-        if os.environ.get("EDB_ALLOW_EXPERIMENTAL", "0") != "1":
-            raise RuntimeError(
-                f"{experimental}: experimental multi-stream switches are gated on GPUs (kernels that "
-                "spin on peer / sibling CTAs are sized for an idle GPU and are not co-residency safe "
-                "next to a second stream); set EDB_ALLOW_EXPERIMENTAL=1 to try them anyway")
-        logger.warning("experimental switches %s enabled (EDB_ALLOW_EXPERIMENTAL=1): not "
-                       "co-residency safe, not part of the measured configuration", experimental)
-    overlap = os.environ.get("EDB_OVERLAP", "0") == "1" and io is not None and ranks is not None \
-        and len(ranks) > 1
-    if overlap:
-        # stream-level overlap instead of in-kernel fusion: plain GEMMs on the compute stream,
-        # collectives on the communication lane
-        info["overlap"] = lowering.overlap_schedule(gm, io, ops)
-    elif (native or fuse_rt is not None) and fuse and io is not None and ranks is not None \
+    if (native or fuse_rt is not None) and fuse and io is not None and ranks is not None \
             and len(ranks) > 1:
         if fuse_rt is None:
             from .runtime import get_runtime
@@ -170,7 +150,7 @@ def _finish(gm, params, buffers, named_states, args, kwargs, ops, native, io=Non
         # buffers of the other dims' collectives.)
         push = ranks is not None and len(ranks) > 1 \
             and os.environ.get("EDB_PUSH_COLL", "1") == "1" and hasattr(ops, "epoch_barrier") \
-            and not overlap and _single_group(gm, ops, ranks)
+            and _single_group(gm, ops, ranks)
         info["symm_bytes"] = lowering.assign_static_buffers(gm, get_runtime(), ops, push=push)
         if push and any(nd.kwargs.get("_push") for nd in gm.graph.nodes if nd.op == "call_function"):
             lowering.ensure_end_barrier(gm, ranks, ops)

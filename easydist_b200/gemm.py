@@ -18,7 +18,6 @@ the share of native GEMMs is visible in `stats()`.
 """
 import torch
 from torch._subclasses.fake_tensor import FakeTensor
-from torch.fx.node import has_side_effect
 
 from . import _lib
 from ._lib import check, i64_array
@@ -106,49 +105,6 @@ def _prepare(t, unit_dim):
     return rowmajor, kmajor, ld
 
 
-class _SideStream:
-    """Second compute stream for GEMMs whose result is not needed right away (weight gradients:
-    `lowering.parallel_wgrad_gemms`, opt-in).  Two persistent GEMM kernels on two streams share the
-    SMs at CTA granularity: the 20 SMs a 128-tile GEMM leaves idle start on the other GEMM's tiles.
-    Fork = the side stream waits for the current one, join = `gemm.join` waits for the event."""
-    stream = None
-
-    def __init__(self, on):
-        self.on = bool(on)
-        self.done = None
-
-    def __enter__(self):
-        if self.on:
-            if _SideStream.stream is None:
-                _SideStream.stream = torch.cuda.Stream()
-            _SideStream.stream.wait_stream(torch.cuda.current_stream())
-            self._ctx = torch.cuda.stream(_SideStream.stream)
-            self._ctx.__enter__()
-        return self
-
-    def __exit__(self, *exc):
-        if self.on:
-            self.done = torch.cuda.Event()
-            self.done.record(_SideStream.stream)
-            self._ctx.__exit__(*exc)
-        return False
-
-
-@has_side_effect
-def join(x):
-    """Make the current stream wait for the side-stream GEMM that produces (the storage of) `x`.
-    Views taken of the result before the join carry the same pending event through `_base`."""
-    t = x
-    while t is not None:
-        pending = getattr(t, "_edb_gemm_pending", None)
-        if pending is not None:
-            torch.cuda.current_stream().wait_event(pending[0])
-            del t._edb_gemm_pending
-            break
-        t = t._base if isinstance(t, torch.Tensor) else None
-    return x
-
-
 def _pf_arrays(pf):
     import ctypes
     items = pf["items"]
@@ -173,7 +129,7 @@ def prefetch_standalone(pf, device):
 EPI_ADD, EPI_GELU_BWD = 1, 2
 
 
-def _launch(a, b, bias, side=0, pf=None, epi=None):
+def _launch(a, b, bias, pf=None, epi=None):
     pa = _prepare(a, 1)
     pb = _prepare(b, 0)
     if pa is None or pb is None:
@@ -186,42 +142,37 @@ def _launch(a, b, bias, side=0, pf=None, epi=None):
     if bias is not None and (N % 8 or bias.data_ptr() % 16 or not bias.is_contiguous()):
         return None
     lib = _lib.load()
-    # operands were staged and the output allocated on the caller's stream; only the kernel forks
     if epi is not None:
         op, aux = epi
         if N % 8 or aux.dtype != torch.bfloat16 or aux.shape != (M, N) or aux.stride(1) != 1 or \
                 aux.stride(0) % 8 or aux.data_ptr() % 16:
             return None
-    with _SideStream(side) as fork:
-        if epi is not None:
-            import ctypes
-            if pf:
-                from .runtime import get_runtime
-                gid = get_runtime().group(pf["group"])
-                k, src, dst, nbytes, stride, sstride = _pf_arrays(pf)
-            else:
-                gid, k, src, dst, nbytes, stride, sstride = 0, 0, None, None, None, None, None
-            check(lib.edb_gemm_epi_bf16(out.data_ptr(), ta.data_ptr(), tb.data_ptr(),
-                                        bias.data_ptr() if bias is not None else None,
-                                        aux.data_ptr(), aux.stride(0), int(op), M, N, K, lda, ldb, ldc,
-                                        1 if a_k else 0, 1 if b_k else 0, gid, k, src, dst, nbytes,
-                                        stride, sstride, _stream(a)))
-            _stats["edb_gemm_epi"] = _stats.get("edb_gemm_epi", 0) + 1
-        elif pf:
-            # the GEMM carries an all-gather prefetch for a later kernel (lowering.prefetch_param_gathers)
+        import ctypes
+        if pf:
             from .runtime import get_runtime
             gid = get_runtime().group(pf["group"])
             k, src, dst, nbytes, stride, sstride = _pf_arrays(pf)
-            check(lib.edb_gemm_pf_bf16(out.data_ptr(), ta.data_ptr(), tb.data_ptr(),
-                                       bias.data_ptr() if bias is not None else None, M, N, K, lda,
-                                       ldb, ldc, 1 if a_k else 0, 1 if b_k else 0, gid, k, src, dst,
-                                       nbytes, stride, sstride, _stream(a)))
         else:
-            check(lib.edb_gemm_bf16(out.data_ptr(), ta.data_ptr(), tb.data_ptr(),
-                                    bias.data_ptr() if bias is not None else None, M, N, K, lda, ldb,
-                                    ldc, 1 if a_k else 0, 1 if b_k else 0, 0, _stream(a)))
-    if fork.on:
-        out._edb_gemm_pending = (fork.done, (ta, tb))
+            gid, k, src, dst, nbytes, stride, sstride = 0, 0, None, None, None, None, None
+        check(lib.edb_gemm_epi_bf16(out.data_ptr(), ta.data_ptr(), tb.data_ptr(),
+                                    bias.data_ptr() if bias is not None else None,
+                                    aux.data_ptr(), aux.stride(0), int(op), M, N, K, lda, ldb, ldc,
+                                    1 if a_k else 0, 1 if b_k else 0, gid, k, src, dst, nbytes,
+                                    stride, sstride, _stream(a)))
+        _stats["edb_gemm_epi"] = _stats.get("edb_gemm_epi", 0) + 1
+    elif pf:
+        # the GEMM carries an all-gather prefetch for a later kernel (lowering.prefetch_param_gathers)
+        from .runtime import get_runtime
+        gid = get_runtime().group(pf["group"])
+        k, src, dst, nbytes, stride, sstride = _pf_arrays(pf)
+        check(lib.edb_gemm_pf_bf16(out.data_ptr(), ta.data_ptr(), tb.data_ptr(),
+                                   bias.data_ptr() if bias is not None else None, M, N, K, lda,
+                                   ldb, ldc, 1 if a_k else 0, 1 if b_k else 0, gid, k, src, dst,
+                                   nbytes, stride, sstride, _stream(a)))
+    else:
+        check(lib.edb_gemm_bf16(out.data_ptr(), ta.data_ptr(), tb.data_ptr(),
+                                bias.data_ptr() if bias is not None else None, M, N, K, lda, ldb,
+                                ldc, 1 if a_k else 0, 1 if b_k else 0, 0, _stream(a)))
     _stats["edb_gemm"] += 1
     if len(_calls) < 8192:
         _calls.append((M, N, K, bool(a_k), bool(b_k), tuple(a.stride()), tuple(b.stride())))
@@ -241,14 +192,13 @@ def _count_unsupported(a, b):
     _stats["aten_mm"] += 1
 
 
-def mm(a, b, *, _side=0, _pf=None):
-    """aten.mm.default(a, b) with bf16 operands on the tcgen05 kernel.  `_side=1`: launched on the
-    side stream; some later `join` of the result (or of a view of it) must precede its first use.
+def mm(a, b, *, _pf=None):
+    """aten.mm.default(a, b) with bf16 operands on the tcgen05 kernel.
     `_pf`: all-gather prefetch carried by this launch ({"group": ranks, "items": [(src_off,
     dst_off, bytes, dst_stride), ...]}, see edb_gemm_pf_bf16)."""
     if isinstance(a, FakeTensor) or isinstance(b, FakeTensor) or a.is_meta:
         return torch.ops.aten.mm.default(a, b)
-    out = _launch(a, b, None, _side, _pf) if _eligible(a, b) else None
+    out = _launch(a, b, None, _pf) if _eligible(a, b) else None
     if out is None:
         if _pf:
             prefetch_standalone(_pf, a.device)  # the gather must happen whoever runs the GEMM
@@ -270,7 +220,7 @@ def mm_add(a, b, res, bias=None, *, _pf=None):
     ok_bias = bias is None or (bias.dim() == 1 and bias.dtype == torch.bfloat16 and
                                bias.shape[0] == b.shape[1])
     if _eligible(a, b) and ok_bias and isinstance(res, torch.Tensor) and res.dim() == 2:
-        out = _launch(a, b, bias, 0, _pf, (EPI_ADD, res))
+        out = _launch(a, b, bias, _pf, (EPI_ADD, res))
         if out is not None:
             return out
     y = mm(a, b, _pf=_pf) if bias is None else addmm(bias, a, b, _pf=_pf)
@@ -283,7 +233,7 @@ def mm_gelu_bwd(a, b, pre, *, _pf=None):
         return torch.ops.aten.gelu_backward.default(torch.ops.aten.mm.default(a, b), pre,
                                                     approximate="tanh")
     if _eligible(a, b) and isinstance(pre, torch.Tensor) and pre.dim() == 2:
-        out = _launch(a, b, None, 0, _pf, (EPI_GELU_BWD, pre))
+        out = _launch(a, b, None, _pf, (EPI_GELU_BWD, pre))
         if out is not None:
             return out
     return torch.ops.aten.gelu_backward.default(mm(a, b, _pf=_pf), pre, approximate="tanh")
@@ -295,11 +245,11 @@ def addmm(bias, a, b, *, _pf=None):
         return torch.ops.aten.addmm.default(bias, a, b)
     if _eligible(a, b) and bias.dim() == 1 and bias.dtype == torch.bfloat16 and \
             bias.shape[0] == b.shape[1]:
-        out = _launch(a, b, bias, 0, _pf)
+        out = _launch(a, b, bias, _pf)
         if out is not None:
             return out
     if _eligible(a, b):
-        out = _launch(a, b, None, 0, _pf)
+        out = _launch(a, b, None, _pf)
         if out is not None:
             return torch.ops.aten.add.Tensor(out, bias)
     if _pf:

@@ -636,71 +636,6 @@ def bucket_small_comm(gm, ops=_default_ops, max_bytes=1 << 20, max_bucket_bytes=
     return done
 
 
-def overlap_schedule(gm, io, ops=_default_ops, prefetch=2):
-    """Stream-level overlap of the DP collectives with compute (opt-in `EDB_OVERLAP=1`; the
-    reference's counterpart is the ordering half of passes/comm_optimize.py:50-141).
-
-      * all-gathers of parameter shards (inputs are placeholders, legal anywhere) are marked
-        `_lane=1` and their *_start hoisted `prefetch` gathers ahead: the weights of the next
-        layers travel while the current layer computes; the *_end stays in front of the first use;
-      * reduce-scatters / all-reduces of gradients are marked `_lane=1` and their *_end sunk to
-        the first reader of the result (the optimizer): gradient reduction overlaps the rest of
-        the backward pass.
-
-    Lane ops run on the communication stream with their own group / op sequence
-    (reshard._Lane); values are unchanged.  Returns {"prefetched": n, "deferred": n}."""
-    graph = gm.graph
-    param_ph = set(io.param_ph)
-    order = {nd: i for i, nd in enumerate(graph.nodes)}
-
-    def pair(st):
-        if len(st.users) != 1:
-            return None
-        end = next(iter(st.users))
-        return end if end.target in ops.COMM_SYNC_FUNCS else None
-
-    def lane(st):
-        kw = dict(st.kwargs)
-        kw["_lane"] = 1
-        st.kwargs = kw
-
-    gathers = []
-    for st in graph.nodes:
-        if st.op == "call_function" and st.target is ops.all_gather_start and st.args[0] in param_ph:
-            end = pair(st)
-            if end is not None and end.users:
-                gathers.append((st, end))
-    # hoist: gather i starts right after the end of gather i - prefetch (never later than it was)
-    for i, (st, end) in enumerate(gathers):
-        lane(st)
-        if i >= prefetch:
-            anchor = gathers[i - prefetch][1]
-            if order[anchor] < order[st]:
-                anchor.append(st)
-        elif i > 0:
-            gathers[i - 1][0].append(st)  # the first `prefetch` gathers all start at the top
-    region = optimizer_region(gm, io)
-    region_set = set(region)
-    deferred = 0
-    order = {nd: i for i, nd in enumerate(graph.nodes)}
-    for st in list(graph.nodes):
-        if st.op != "call_function" or st.target not in (ops.reduce_scatter_start,
-                                                         ops.all_reduce_start):
-            continue
-        end = pair(st)
-        if end is None or not end.users:
-            continue
-        if st not in region_set:  # only gradient collectives (downstream of the final grads)
-            continue
-        first = min(end.users, key=lambda u: order[u])
-        lane(st)
-        first.prepend(end)
-        deferred += 1
-    graph.lint()
-    gm.recompile()
-    return {"prefetched": len(gathers), "deferred": deferred}
-
-
 def _is_functional_foreach(target):
     schema = getattr(target, "_schema", None)
     return schema is not None and schema.name.startswith("aten::_foreach_") and \
@@ -892,11 +827,10 @@ def assign_static_buffers(gm, rt, ops=_default_ops, push=False):
         if node.op != "call_function" or node.target not in ops.COMM_FUNCS:
             continue
         x = node.args[0].meta["val"]
-        lane = bool(node.kwargs.get("_lane"))
         if node.target is ops.all_gather_start:
             need = [_nbytes(node.meta["val"])]
         elif node.target is ops.all_reduce_start:
-            if push and not lane:
+            if push:
                 grp = node.args[2]
                 need = list(ops.all_reduce_push_sizes(_nbytes(x), x.numel(), x.element_size(),
                                                       len(grp), oneshot))
@@ -910,7 +844,7 @@ def assign_static_buffers(gm, rt, ops=_default_ops, push=False):
         total += sum(need)
         kw = dict(node.kwargs)
         kw["_buf"] = (bufs[0].offset, need[0]) + tuple(b.offset for b in bufs[1:])
-        if push and not lane:
+        if push:
             kw["_push"] = 1
         node.kwargs = kw
     gm.recompile()
@@ -1053,59 +987,6 @@ def fuse_optimizer_updates(gm):
     return n
 
 
-_VIEW_ONLY = None
-
-
-def parallel_wgrad_gemms(gm):
-    """Opt-in (`EDB_GEMM_SIDE=1`): GEMMs whose result is first *computed on* much later (weight
-    gradients: read by the optimizer) are launched on a second compute stream and joined right in
-    front of that first reader.  Two persistent GEMM kernels then share the SMs at CTA granularity,
-    which fills the wave a 128-tile GEMM leaves 14 % empty, and hides launch gaps.  Only metadata
-    ops (t / view / permute ...) may touch the result before the join.  Returns the number of GEMMs
-    moved."""
-    global _VIEW_ONLY
-    from . import gemm
-    if _VIEW_ONLY is None:
-        _VIEW_ONLY = {aten.t.default, aten.view.default, aten._unsafe_view.default,
-                      aten.transpose.int, aten.permute.default, aten.alias.default,
-                      aten.detach.default, aten.unsqueeze.default, aten.squeeze.dim}
-    graph = gm.graph
-    nodes = list(graph.nodes)
-    order = {n: i for i, n in enumerate(nodes)}
-    moved = 0
-    # latest first: of a (data-gradient, weight-gradient) pair only the one whose reader is far
-    # away moves; a GEMM that only has moved GEMMs before its reader would overlap with nothing
-    for node in reversed(nodes):
-        if node.op != "call_function" or node.target is not gemm.mm or node.kwargs:
-            continue
-        consumers, frontier, seen = [], [node], {node}
-        while frontier:
-            cur = frontier.pop()
-            for u in cur.users:
-                if u in seen:
-                    continue
-                seen.add(u)
-                if u.op == "call_function" and u.target in _VIEW_ONLY:
-                    frontier.append(u)
-                else:
-                    consumers.append(u)
-        if not consumers:
-            continue
-        first = min(consumers, key=lambda u: order[u])
-        between = nodes[order[node] + 1:order[first]]
-        if not any(b.op == "call_function" and b.target in (gemm.mm, gemm.addmm)
-                   and not b.kwargs.get("_side") for b in between):
-            continue  # nothing on the main stream to overlap with
-        node.kwargs = {"_side": 1}
-        with graph.inserting_before(first):
-            graph.call_function(gemm.join, args=(node,))
-        moved += 1
-    if moved:
-        graph.lint()
-        gm.recompile()
-    return moved
-
-
 def fuse_gemm_epilogues(gm):
     """Elementwise neighbours of the native GEMMs move into their epilogues (edb_gemm_epi_bf16):
 
@@ -1131,7 +1012,7 @@ def fuse_gemm_epilogues(gm):
             chain.append(nd)
             nd = nd.args[0]
         if isinstance(nd, Node) and nd.op == "call_function" and nd.target in (gemm.mm, gemm.addmm) \
-                and len(nd.users) == 1 and not nd.kwargs.get("_side"):
+                and len(nd.users) == 1:
             return nd, chain
         return None, chain
 
@@ -1275,8 +1156,6 @@ def dispatch_compute(gm):
                 node.kwargs = {"_pf": node.meta["edb_pf"]}
             n += 1
     gm.recompile()
-    if os.environ.get("EDB_GEMM_SIDE", "0") == "1":
-        n += parallel_wgrad_gemms(gm)
     if os.environ.get("EDB_FUSE_EPILOGUE", "1") == "1":
         n += fuse_gemm_epilogues(gm)
     return n

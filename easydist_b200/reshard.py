@@ -69,61 +69,10 @@ def _norm_dim(dim, ndim):
     return dim + ndim if dim < 0 else dim
 
 
-def _group(group, lane=0):
+def _group(group):
     rt = get_runtime()
-    gid = rt.group(group, lane=lane)
+    gid = rt.group(group)
     return rt, gid, rt.group_size(gid), rt.group_index(gid)
-
-
-class _Lane:
-    """Communication lane (`_lane=1` on a *_start op, set by lowering.overlap_schedule): the kernel
-    is launched on a side stream that first waits for the current stream, so it overlaps whatever
-    the compute stream does next; the matching *_end makes the consumer stream wait for it
-    (what `wait_tensor` is for the reference's funcol ops, sharding.py:101-102).  Everything is
-    event-based, hence capturable in a CUDA graph as a fork/join.  Lane kernels run with one CTA
-    per SM so that their spinning CTAs stay co-resident next to a compute kernel."""
-    stream = None
-    ctas_per_sm = 1
-
-    def __init__(self, on):
-        self.on = bool(on)
-        self.done = None
-
-    def __enter__(self):
-        if self.on:
-            cur = torch.cuda.current_stream()
-            if _Lane.stream is None:
-                _Lane.stream = torch.cuda.Stream()
-            _Lane.stream.wait_stream(cur)
-            self._ctx = torch.cuda.stream(_Lane.stream)
-            self._ctx.__enter__()
-            rt = get_runtime()
-            self._saved = rt.get_option("copy_ctas_per_sm")
-            rt.set_option("copy_ctas_per_sm", _Lane.ctas_per_sm)
-        return self
-
-    def __exit__(self, *exc):
-        if self.on:
-            get_runtime().set_option("copy_ctas_per_sm", self._saved)
-            self.done = torch.cuda.Event()
-            self.done.record(_Lane.stream)
-            self._ctx.__exit__(*exc)
-        return False
-
-    def tag(self, out, *keep):
-        """Attach the completion event (and the tensors the kernel still reads) to `out`."""
-        if self.on:
-            out._edb_pending = (self.done, keep)
-        return out
-
-
-def _join(t):
-    """*_end: the current stream waits for the lane kernel that produces `t` (no-op otherwise)."""
-    pending = getattr(t, "_edb_pending", None)
-    if pending is not None:
-        torch.cuda.current_stream().wait_event(pending[0])
-        del t._edb_pending
-    return t
 
 
 def _buffers(rt, _buf, sizes):
@@ -144,7 +93,7 @@ def all_reduce_push_sizes(nbytes, numel, elem_size, n, oneshot_bytes):
 
 
 def all_reduce_start(self: torch.Tensor, reduceOp: str, group: List[int], tag: str = "", *,
-                     _buf=None, _lane=0, _push=0):
+                     _buf=None, _push=0):
     """P(op) -> R. Reference: sharding.py:94-98 (c10d_functional.all_reduce).
     `_push=1` (set by lowering.assign_static_buffers for graphs that end with an epoch barrier):
     the push protocol, _buf = (receive offset, size, result offset); the result is a view of the
@@ -152,7 +101,7 @@ def all_reduce_start(self: torch.Tensor, reduceOp: str, group: List[int], tag: s
     if _is_fake(self):
         return torch.empty_like(self, memory_format=torch.contiguous_format)
     _require_cuda(self, "all_reduce_start")
-    rt, gid, n, _ = _group(group, _lane)
+    rt, gid, n, _ = _group(group)
     x = self.contiguous()
     if _push and _buf is not None and n > 1 and x.numel() > 0:
         recv_off, out_off = int(_buf[0]), int(_buf[2])
@@ -166,31 +115,28 @@ def all_reduce_start(self: torch.Tensor, reduceOp: str, group: List[int], tag: s
         return out
     two_shot = n > 1 and nbytes > rt.get_option("allreduce_oneshot_bytes")
     sizes = [nbytes, nbytes] if two_shot else [nbytes]
-    static = False
     if n > 1:
-        bufs, static = _buffers(rt, _buf, sizes)
+        bufs, _ = _buffers(rt, _buf, sizes)
         s1 = bufs[0].offset
         s2 = bufs[1].offset if two_shot else 0
     else:
         s1 = s2 = 0
-    with _Lane(_lane and n > 1 and static) as lane:
-        check(rt.lib.edb_all_reduce(gid, out.data_ptr(), s1, s2, x.data_ptr(), x.numel(),
-                                    _dtype_code(x, "all_reduce_start"),
-                                    _redop(reduceOp, "all_reduce_start"), rt.stream()))
-    return lane.tag(out, x)
+    check(rt.lib.edb_all_reduce(gid, out.data_ptr(), s1, s2, x.data_ptr(), x.numel(),
+                                _dtype_code(x, "all_reduce_start"),
+                                _redop(reduceOp, "all_reduce_start"), rt.stream()))
+    return out
 
 
 def all_reduce_end(self: torch.Tensor, reduceOp: str, group: List[int], tag: str = ""):
-    """Reference: sharding.py:101-102 (wait_tensor). Stream-ordered here: identity, unless the
-    start ran on the communication lane."""
-    return _join(self)
+    """Reference: sharding.py:101-102 (wait_tensor). Identity: the start is stream-ordered."""
+    return self
 
 
 # ---- all_gather --------------------------------------------------------------------------------------
 
 
 def all_gather_start(self: torch.Tensor, gather_dim: int, group: List[int], tag: str = "", *,
-                     _buf=None, _lane=0, _push=0):
+                     _buf=None, _push=0):
     """S(gather_dim) -> R. Reference: sharding.py:105-111 gathers along dim 0 and leaves the
     chunk+cat to all_gather_end (:114-119); here the result is already laid out along
     `gather_dim`."""
@@ -202,25 +148,22 @@ def all_gather_start(self: torch.Tensor, gather_dim: int, group: List[int], tag:
     if _is_fake(self):
         return self.new_empty(out_shape)
     _require_cuda(self, "all_gather_start")
-    rt, gid, n, _ = _group(group, _lane)
+    rt, gid, n, _ = _group(group)
     x = self.contiguous()
     nbytes = x.numel() * x.element_size() * n
     if nbytes == 0:
         return x.new_empty(out_shape)
     (buf,), static = _buffers(rt, _buf, [nbytes])
-    # the lane needs a buffer of its own until *_end: only with static buffers
-    with _Lane(_lane and n > 1 and static) as lane:
-        fn = rt.lib.edb_all_gather_push if (_push and static and not _lane) else rt.lib.edb_all_gather
-        check(fn(gid, buf.offset, x.data_ptr(), i64_array(x.shape), ndim, dim, x.element_size(),
-                 rt.stream()))
-        out = buf.tensor(x.dtype, out_shape)
-        out = out if static else out.clone()
-    return lane.tag(out, x)
+    fn = rt.lib.edb_all_gather_push if (_push and static) else rt.lib.edb_all_gather
+    check(fn(gid, buf.offset, x.data_ptr(), i64_array(x.shape), ndim, dim, x.element_size(),
+             rt.stream()))
+    out = buf.tensor(x.dtype, out_shape)
+    return out if static else out.clone()
 
 
 def all_gather_end(self: torch.Tensor, gather_dim: int, group: List[int], tag: str = ""):
     """Reference: sharding.py:114-119. Identity: all_gather_start already produced the layout."""
-    return _join(self)
+    return self
 
 
 # ---- local ops ---------------------------------------------------------------------------------------
@@ -274,7 +217,7 @@ def copy_wrapper(self, other):
 
 def reduce_scatter_start(self: torch.Tensor, reduceOp: str, scatter_dim: int, group: List[int],
                          tag: str = "", *, _buf=None, _scale: float = 1.0, _out_dtype=None,
-                         _lane=0, _push=0):
+                         _push=0):
     """P(op) -> S(scatter_dim). Reference: sharding.py:130-144 (pre-permute copy for dim != 0 and
     reduce_scatter_tensor). `_scale`/`_out_dtype` fuse the gradient scale / cast into the kernel."""
     n = len(group)
@@ -288,9 +231,9 @@ def reduce_scatter_start(self: torch.Tensor, reduceOp: str, scatter_dim: int, gr
     if _is_fake(self):
         return self.new_empty(out_shape, dtype=out_dtype)
     _require_cuda(self, "reduce_scatter_start")
-    rt, gid, n, _ = _group(group, _lane)
+    rt, gid, n, _ = _group(group)
     x = self.contiguous()
-    out = x.new_empty(out_shape, dtype=out_dtype)  # on the consumer's stream, also for lane ops
+    out = x.new_empty(out_shape, dtype=out_dtype)
     nbytes = x.numel() * x.element_size()
     if nbytes == 0:
         return out
@@ -298,21 +241,18 @@ def reduce_scatter_start(self: torch.Tensor, reduceOp: str, scatter_dim: int, gr
     if n > 1:
         (buf,), static = _buffers(rt, _buf, [nbytes])
         stage = buf.offset
-    with _Lane(_lane and n > 1 and static) as lane:
-        fn = rt.lib.edb_reduce_scatter_push if (_push and static and not _lane) \
-            else rt.lib.edb_reduce_scatter
-        check(fn(gid, out.data_ptr(), stage, x.data_ptr(),
-                 i64_array(x.shape), ndim, dim, _dtype_code(x, "reduce_scatter_start"),
-                 _redop(reduceOp, "reduce_scatter_start"), float(_scale),
-                 _TORCH_DTYPE_CODE[out_dtype], rt.stream()))
-    return lane.tag(out, x)
+    fn = rt.lib.edb_reduce_scatter_push if (_push and static) else rt.lib.edb_reduce_scatter
+    check(fn(gid, out.data_ptr(), stage, x.data_ptr(),
+             i64_array(x.shape), ndim, dim, _dtype_code(x, "reduce_scatter_start"),
+             _redop(reduceOp, "reduce_scatter_start"), float(_scale),
+             _TORCH_DTYPE_CODE[out_dtype], rt.stream()))
+    return out
 
 
 def reduce_scatter_end(self: torch.Tensor, reduceOp: str, scatter_dim: int, group: List[int],
                        tag: str = ""):
-    """Reference: sharding.py:147-152 (wait_tensor). Identity, unless the start ran on the
-    communication lane."""
-    return _join(self)
+    """Reference: sharding.py:147-152 (wait_tensor). Identity: the start is stream-ordered."""
+    return self
 
 
 # ---- all_to_all --------------------------------------------------------------------------------------

@@ -133,19 +133,14 @@ class Runtime:
                                     f"symmetric heap diverged across ranks after compilation: {marks}")
             dist.barrier(group=getattr(self, "_pg", None))
 
-    def group(self, ranks, slot=None, lane=0):
+    def group(self, ranks, slot=None):
         """gid of the group of global `ranks` (mesh-dim order); created on first use.
 
         Slots are assigned in creation order; SPMD programs create their groups in the same
         order on every member (mesh dim 0, 1, ... then the world group), which keeps them equal.
-        `lane` > 0 names a second group over the same ranks with its own flag block and op
-        sequence: collectives issued on the communication stream (reshard `_lane=1`) are ordered
-        among themselves on every rank, but not against the compute stream's ops.
         """
-        key = tuple(int(r) for r in ranks)
-        if lane:
-            key = ("lane", int(lane)) + key
-        gid = self._groups.get(key)
+        members = tuple(int(r) for r in ranks)
+        gid = self._groups.get(members)
         if gid is not None:
             return gid
         if not self._attached:
@@ -153,11 +148,10 @@ class Runtime:
         if slot is None:
             slot = len(self._groups)
         out = c_int()
-        members = tuple(int(r) for r in ranks)
         check(self.lib.edb_group_create(_lib.int_array(members), len(members), int(slot), byref(out)))
         n, me = c_int(), c_int()
         check(self.lib.edb_group_info(out.value, byref(n), byref(me)))
-        self._groups[key] = out.value
+        self._groups[members] = out.value
         self._group_meta[out.value] = (n.value, me.value, members)
         return out.value
 

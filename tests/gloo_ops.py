@@ -43,7 +43,7 @@ _OPS = {"sum": dist.ReduceOp.SUM, "max": dist.ReduceOp.MAX, "min": dist.ReduceOp
         "avg": dist.ReduceOp.SUM}
 
 
-def all_reduce_start(self, reduceOp: str, group: List[int], tag: str = "", *, _buf=None, _lane=0):
+def all_reduce_start(self, reduceOp: str, group: List[int], tag: str = "", *, _buf=None):
     if _fake(self):
         return torch.empty_like(self)
     out = self.contiguous().clone()
@@ -58,7 +58,7 @@ def all_reduce_end(self, reduceOp, group, tag=""):
     return self
 
 
-def all_gather_start(self, gather_dim: int, group: List[int], tag: str = "", *, _buf=None, _lane=0):
+def all_gather_start(self, gather_dim: int, group: List[int], tag: str = "", *, _buf=None):
     n = len(group)
     shape = list(self.shape)
     shape[gather_dim] *= n
@@ -82,7 +82,7 @@ def copy_wrapper(self, other):
 
 
 def reduce_scatter_start(self, reduceOp: str, scatter_dim: int, group: List[int], tag: str = "", *,
-                         _buf=None, _scale=1.0, _out_dtype=None, _lane=0):
+                         _buf=None, _scale=1.0, _out_dtype=None):
     n = len(group)
     assert self.size(scatter_dim) % n == 0
     shape = list(self.shape)

@@ -671,59 +671,6 @@ def bench_fused(rank, world, group):
                   f"(wgrad gemm alone {t_wg:.1f}us)", flush=True)
 
 
-def run_lane(rank, world, group):
-    """EXPERIMENTAL (EDB_TEST_EXPERIMENTAL=1): collectives on the communication lane (`_lane=1`,
-    side stream + own group) overlapped with compute-stream GEMMs and compute-lane collectives;
-    eager and from a replayed CUDA graph; bit-exact vs the oracle."""
-    from easydist_b200 import gemm
-    rt = runtime.get_runtime()
-    rows = 256
-    x = torch.zeros(rows * world, 512, device="cuda")
-    buf_ag = rt.alloc(x.numel() * 4 * world)
-    buf_rs = rt.alloc(x.numel() * 4)
-    buf_ar = rt.alloc(x.numel() * 4)
-    buf_ar2 = rt.alloc(x.numel() * 4)  # second stage of the two-shot all-reduce
-    a = torch.randn(2048, 2048, device="cuda").bfloat16()
-    b = torch.randn(2048, 2048, device="cuda").bfloat16()
-
-    def step():
-        g = reshard.all_gather_start(x, 0, group, _buf=(buf_ag.offset, buf_ag.nbytes), _lane=1)
-        r = reshard.reduce_scatter_start(x, "sum", 0, group, _buf=(buf_rs.offset, buf_rs.nbytes),
-                                         _lane=1)
-        c = gemm.mm(a, b)                                   # compute stream, overlaps the lane
-        s = reshard.all_reduce_start(x, "max", group,  # compute lane, concurrent with the lane ops
-                                     _buf=(buf_ar.offset, buf_ar.nbytes, buf_ar2.offset))
-        c2 = gemm.mm(c, b)
-        g = reshard.all_gather_end(g, 0, group)
-        r = reshard.reduce_scatter_end(r, "sum", 0, group)
-        return g.clone(), r.clone(), s.clone(), c2
-
-    def expect(vals):
-        full = np.concatenate([np.full((rows * world, 512), v, np.float32) for v in vals])
-        red = np.full((rows, 512), float(sum(vals)), np.float32)
-        return full, red, np.full((rows * world, 512), float(max(vals)), np.float32)
-
-    n_ok = 0
-    for it in range(3):
-        x.fill_(float(rank + 1 + it))
-        outs = step()
-        torch.cuda.synchronize()
-        for o, w in zip(outs[:3], expect([r_ + 1 + it for r_ in range(world)])):
-            check_equal(o, w, f"lane eager {it}")
-            n_ok += 1
-    graph = torch.cuda.CUDAGraph()
-    with torch.cuda.graph(graph):
-        outs = step()
-    for it in range(4):
-        x.fill_(float(rank + 3 + it))
-        graph.replay()
-        torch.cuda.synchronize()
-        for o, w in zip(outs[:3], expect([r_ + 3 + it for r_ in range(world)])):
-            check_equal(o, w, f"lane graph {it}")
-            n_ok += 1
-    return n_ok
-
-
 def run_auto_bundle(rank, world):
     """Auto-SPMD on real GPUs: graph + plan solved by the unmodified reference (recorded in
     tests/golden/auto_foo_mesh*.json), lowered by easydist_b200.lowering.sharding_transform and
@@ -985,8 +932,6 @@ def main():
     n += run_push_cases(rank, world, group)
     n += run_auto_bundle(rank, world)
     n += run_train_parity(rank, world)
-    if os.environ.get("EDB_TEST_EXPERIMENTAL") == "1":
-        n += run_lane(rank, world, group)
     if world in (2, 4, 8) and os.environ.get("EDB_SKIP_C1") != "1":
         # SURVEY.md config 1 (the reference's examples/torch/gpt_train.py model, fp32) in AUTO-SPMD
         # mode with the plans the reference's solver produced, on real GPUs: outputs, every parameter

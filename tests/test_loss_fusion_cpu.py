@@ -127,40 +127,3 @@ def test_sgd_momentum_triple_is_fused_and_matches_unfused(opt_kw, expect):
     got, want = compiled.named_parameters(), plain.named_parameters()
     for name in want:
         assert torch.equal(got[name], want[name]), name
-
-
-def test_weight_gradient_gemms_move_to_the_side_stream_with_a_join_before_first_use():
-    """lowering.parallel_wgrad_gemms (opt-in EDB_GEMM_SIDE=1): every GEMM whose result is first
-    computed on after another GEMM (the weight gradients, read by the optimizer) gets `_side=1` and a
-    `gemm.join` right in front of that reader; only metadata ops sit between the GEMM and its join;
-    results are unchanged (on CPU the GEMMs take their ATen branch)."""
-    from easydist_b200 import gemm
-    set_device_mesh([0], ["dp"], rank=0)
-    cfg = workloads.GPT2_CONFIGS["gpt2-tiny"]
-    torch.manual_seed(0)
-    model = workloads.GPT2(cfg).bfloat16()
-    ref = workloads.GPT2(cfg).bfloat16()
-    ref.load_state_dict(model.state_dict())
-    opt = torch.optim.SGD(model.parameters(), lr=0.05, momentum=0.9, foreach=True)
-    ropt = torch.optim.SGD(ref.parameters(), lr=0.05, momentum=0.9, foreach=True)
-    tok, tgt = workloads.synthetic_tokens(cfg, 2, 32, 0)
-    compiled = api._compile_dp(workloads.gpt2_train_step, "ddp", "fake", (tok, tgt, model, opt), {},
-                               ops=gloo_ops, native=False)
-    gm = compiled.graph
-    lowering.dispatch_compute(gm)
-    moved = lowering.parallel_wgrad_gemms(gm)
-    nodes = list(gm.graph.nodes)
-    pos = {n: i for i, n in enumerate(nodes)}
-    side = [n for n in nodes if n.op == "call_function" and n.target is gemm.mm and n.kwargs.get("_side")]
-    joins = [n for n in nodes if n.op == "call_function" and n.target is gemm.join]
-    # 2 layers x 4 Linear weight gradients + the LM head's
-    assert moved == len(side) == len(joins) == 9, (moved, len(side), len(joins))
-    for j in joins:
-        src = j.args[0]
-        assert src.kwargs.get("_side") == 1 and pos[src] < pos[j]
-        users_before_join = [u for u in nodes[pos[src] + 1:pos[j]] if src in u.all_input_nodes]
-        assert all(u.target in lowering._VIEW_ONLY for u in users_before_join)
-    for _ in range(2):
-        l = compiled(tok, tgt, model, opt)
-        l_ref = workloads.gpt2_train_step(tok, tgt, ref, ropt)
-        assert torch.allclose(l.float(), l_ref.detach().float(), rtol=1e-2, atol=1e-3)

@@ -1,7 +1,7 @@
 """Host side of easydist_b200.reshard with the C-ABI mocked out: which entry point each of the
 reference-signature callables reaches, with which arguments (shapes, dims, dtype / redop codes,
-symmetric offsets, group ids incl. the communication lane), what it returns, and the errors it
-raises — no GPU, no compute.  (The kernels behind the entry points are checked by the -m gpu tests.)"""
+symmetric offsets, group ids), what it returns, and the errors it raises — no GPU, no compute.
+(The kernels behind the entry points are checked by the -m gpu tests.)"""
 import ctypes
 
 import pytest
@@ -34,11 +34,10 @@ class _FakeRuntime:
         self.slab = torch.zeros(1 << 22, dtype=torch.uint8)
         self.groups = {}
         self._ring = 1 << 16
-        self.options = {"allreduce_oneshot_bytes": 512 * 1024, "copy_ctas_per_sm": 4}
+        self.options = {"allreduce_oneshot_bytes": 512 * 1024}
 
-    def group(self, ranks, slot=None, lane=0):
-        key = (lane,) + tuple(ranks)
-        return self.groups.setdefault(key, len(self.groups))
+    def group(self, ranks, slot=None):
+        return self.groups.setdefault(tuple(ranks), len(self.groups))
 
     def group_size(self, gid):
         return self.world
@@ -48,9 +47,6 @@ class _FakeRuntime:
 
     def get_option(self, name):
         return self.options[name]
-
-    def set_option(self, name, value):
-        self.options[name] = value
 
     def stream(self):
         return ctypes.c_void_p(0)
@@ -100,6 +96,7 @@ def test_reduce_scatter_codes_scale_and_divisibility(rt):
     assert args[7] == _lib.DTYPE_CODES["bfloat16"] and args[8] == _lib.REDOP_CODES["avg"]
     assert args[9] == 0.5 and args[10] == _lib.DTYPE_CODES["float32"]
     assert out.shape == (4, 3) and out.dtype == torch.float32
+    assert reshard.reduce_scatter_end(out, "avg", 1, [0, 1]) is out
     with pytest.raises(AssertionError):                          # sharding.py:136-137
         reshard.reduce_scatter_start(torch.ones(3, 5), "sum", 0, [0, 1])
     with pytest.raises(_lib.EdbError):
@@ -108,7 +105,8 @@ def test_reduce_scatter_codes_scale_and_divisibility(rt):
 
 def test_all_reduce_one_and_two_shot_buffers(rt):
     small = torch.ones(1024)
-    reshard.all_reduce_start(small, "sum", [0, 1])
+    out = reshard.all_reduce_start(small, "sum", [0, 1])
+    assert reshard.all_reduce_end(out, "sum", [0, 1]) is out
     big = torch.ones(1 << 18)                                    # 1 MiB > one-shot threshold
     reshard.all_reduce_start(big, "max", [0, 1])
     (_, a_small), (_, a_big) = rt.lib.calls
@@ -117,20 +115,6 @@ def test_all_reduce_one_and_two_shot_buffers(rt):
     assert a_big[7] == _lib.REDOP_CODES["max"]
     with pytest.raises(_lib.EdbError):
         reshard.all_reduce_start(torch.ones(4, dtype=torch.bool), "sum", [0, 1])
-
-
-def test_lane_ops_use_their_own_group_and_default_ops_do_not(rt):
-    x = torch.ones(8, 8)
-    reshard.all_reduce_start(x, "sum", [0, 1])
-    gid_default = rt.lib.calls[-1][1][0]
-    assert rt.groups == {(0, 0, 1): gid_default}
-    # a lane op without static buffers stays on the caller's stream (no CUDA needed here) but
-    # already addresses the lane's group: its own flag block and op sequence
-    reshard.all_reduce_start(x, "sum", [0, 1], _lane=1)
-    assert rt.lib.calls[-1][1][0] == rt.groups[(1, 0, 1)] != gid_default
-    out = reshard.reduce_scatter_start(x, "sum", 0, [0, 1], _lane=1)
-    assert not hasattr(out, "_edb_pending")
-    assert reshard.reduce_scatter_end(out, "sum", 0, [0, 1]) is out
 
 
 def test_scatter_wrapper_chunks_like_torch_chunk(rt):
@@ -161,9 +145,9 @@ def test_product_path_has_no_cpu_fallback():
         reshard.scatter_wrapper(torch.ones(2, 2), 2, 0, 0)
 
 
-def test_runtime_group_registry_and_lanes():
-    """Runtime.group: one C-ABI group per (lane, ranks); slots follow creation order; the lane's
-    group has the same members but its own gid / slot (flag block, op sequence)."""
+def test_runtime_group_registry():
+    """Runtime.group: one C-ABI group per set of ranks, created on first use and cached; slots
+    follow creation order."""
     from easydist_b200.runtime import Runtime
 
     class Lib:
@@ -183,10 +167,11 @@ def test_runtime_group_registry_and_lanes():
     rt = object.__new__(Runtime)
     rt.lib, rt._groups, rt._group_meta, rt._attached = Lib(), {}, {}, True
     g0 = rt.group([0, 1])
-    assert rt.group((0, 1)) == g0 and rt.group([0, 1], lane=0) == g0        # cached, lane 0 = default
-    g1 = rt.group([0, 1], lane=1)
-    g2 = rt.group([0, 2])
+    assert rt.group((0, 1)) == g0                                            # cached
+    g1 = rt.group([0, 2])
+    g2 = rt.group([0, 1, 2, 3])
     assert len({g0, g1, g2}) == 3
-    assert rt.lib.created == [([0, 1], 0), ([0, 1], 1), ([0, 2], 2)]
+    assert rt.lib.created == [([0, 1], 0), ([0, 2], 1), ([0, 1, 2, 3], 2)]
     assert rt.group_size(g1) == 2 and rt.group_index(g1) == 1
-    assert rt.group([0, 1], lane=1) == g1
+    assert rt.group_size(g2) == 4 and rt.group_index(g2) == 1
+    assert rt.group([0, 2]) == g1 and rt.group([0, 1, 2, 3]) == g2
